@@ -540,21 +540,12 @@ def clock_window(cx):
     return cx.sampler.window() if cx.sampler else _NullWindow()
 
 
-def percentile(xs, q):
-    xs = sorted(xs)
-    if not xs:
-        return None
-    k = (len(xs) - 1) * q
-    lo, hi = int(math.floor(k)), int(math.ceil(k))
-    return xs[lo] + (xs[hi] - xs[lo]) * (k - lo)
-
-
-def measure_device(cx, args, env_id, n, K, W, ring_arg=0, min_region_s=0.05):
+def measure_device(cx, args, env_id, n, K, W, ring_arg=0):
     """`value`: inputs resident in HBM.  A ring of independent n-env batches (footprint > 2 x L2 for the HBM-bound families)
-    is stepped round-robin, one fused launch per bench step.  W plain warm-up launches, then ONE CUDA graph that starts at
-    the ring position after the warm-up and holds q consecutive K-step segments (q*K a multiple of the ring, >= ~10 ms), so
-    replaying it continues the round-robin and every timed launch finds its batch evicted from L2.  The graph is replayed
-    until the timed region is >= 50 ms (CUDA events on the launch stream around every replay; max over ranks)."""
+    is stepped round-robin, one fused launch per bench step, and the steps are ordered so that every timed launch finds
+    its batch evicted from L2.  After the set-up, exactly K step launches are timed: one CUDA graph holds the W warm-up
+    launches, a CUDA event, the K launches and a second event (max over ranks).  `outputs` is what the last timed step
+    returned to its caller (device tensors the graph replay writes)."""
     import gymnasium_b200
 
     torch, dev, rank = cx.torch, cx.dev, cx.rank
@@ -576,69 +567,88 @@ def measure_device(cx, args, env_id, n, K, W, ring_arg=0, min_region_s=0.05):
 
     def launch(i):  # one bench step = one fused step launch on the next batch of the ring
         j = i % ring
-        envs[j].step(acts[j][(i // ring) % T])
-
-    def capture(start, count):
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
-            for i in range(start, start + count):
-                launch(i)
-        return g
+        return envs[j].step(acts[j][(i // ring) % T])
 
     burn = BURN_IN.get(env_id, 0)
-    for i in range(ring * (1 + burn)):  # every code path once + the steady-state mix of a physics family (set-up, untimed)
+    setup = ring * (1 + burn)
+    for i in range(setup):  # every code path once + the steady-state mix of a physics family (set-up, untimed)
         launch(i)
-    for i in range(W):  # the W warm-up launches; the timed graph starts at the ring position right after them
+    # ONE graph: the W warm-up launches (ending on the last batch of the ring), an event, the K timed launches from the
+    # first batch, an event.  The events are nodes of the graph, so no launch boundary or host gap falls in the window.
+    a, b = (torch.cuda.Event(enable_timing=True, external=True) for _ in range(2))
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        for i in range(setup - W, setup):
+            launch(i)
+        a.record()
+        for i in range(setup, setup + K):
+            outputs = launch(i)
+        b.record()
+    g.replay()  # uploads the graph (set-up, untimed)
+    # `pad` set-up launches continue the round-robin up to the batch before the warm-up's first, so that every timed
+    # launch finds its batch the least recently stepped one
+    pad = -(W + K) % ring
+    for i in range(setup + K, setup + K + pad):
         launch(i)
-    torch.cuda.synchronize()
-    s0 = W
-    Kc = K if K <= 4096 else ring * T
-    base = Kc * ring // math.gcd(Kc, ring)
-    g = capture(s0, base)
-    g.replay()
-    torch.cuda.synchronize()
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    a.record()
-    g.replay()
-    b.record()
-    torch.cuda.synchronize()
-    t_base = max_over_ranks(cx, a.elapsed_time(b) * 1e-3)
-    q = max(1, min(math.ceil(0.010 / t_base), max(1, 60000 // base)))
-    if q > 1:
-        del g
-        g = capture(s0, base * q)
-        g.replay()  # uploads the graph; also >= W further untimed launches
-    M = base * q
-    replays = int(min(2000, max(5, math.ceil(min_region_s / (t_base * q)), math.ceil(K / M))))
-    replays = int(max_over_ranks(cx, float(replays)))
-    ev = [torch.cuda.Event(enable_timing=True) for _ in range(replays + 1)]
     sync_all(cx)
     with clock_window(cx):
         sync_all(cx)
-        ev[0].record()
-        for r in range(replays):
-            g.replay()
-            ev[r + 1].record()
+        g.replay()
         sync_all(cx)
-    elapsed = max_over_ranks(cx, ev[0].elapsed_time(ev[-1]) * 1e-3)
-    per_step_ms = [ev[r].elapsed_time(ev[r + 1]) / M for r in range(replays)]
-    timed = replays * M
+    elapsed = max_over_ranks(cx, a.elapsed_time(b) * 1e-3)
     del g
     reset_frac = float(torch.stack([(e._ctrl < 0).float().mean() for e in envs]).mean().item())
     cold = ring * foot > 2 * cx.info["l2_bytes"]
     return {
-        "value": cx.world * timed * n / elapsed, "elapsed_s": elapsed, "timed_steps": timed, "graph_launches": M,
-        "replays": replays, "reps_of_K": timed / K, "ms_per_step": elapsed / timed * 1e3,
-        "ms_per_step_p50": percentile(per_step_ms, 0.5), "ms_per_step_p95": percentile(per_step_ms, 0.95),
-        "ms_per_step_min": min(per_step_ms), "ring": ring, "foot": foot, "reset_frac": reset_frac, "envs": envs,
-        "acts": acts,
+        "value": cx.world * K * n / elapsed, "elapsed_s": elapsed, "timed_steps": K, "graph_launches": W + K,
+        "ms_per_step": elapsed / K * 1e3, "ring": ring, "foot": foot, "reset_frac": reset_frac, "envs": envs,
+        "acts": acts, "outputs": outputs,
         "l2_policy": (f"inputs larger than L2: ring of {ring} independent {n}-env batches ({ring * foot / 1e6:.0f} MB > 2 x "
-                      f"{cx.info['l2_bytes'] / 1e6:.0f} MB L2) stepped round-robin; the timed graph starts at the ring position "
-                      f"after the warm-up launches and its length is a multiple of the ring, so no timed launch is L2-warm"
+                      f"{cx.info['l2_bytes'] / 1e6:.0f} MB L2) stepped round-robin; the timed launches step the batches "
+                      f"in least-recently-stepped order, so no timed launch is L2-warm"
                       if cold else
                       f"ring of {ring} independent {n}-env batches ({ring * foot / 1e6:.0f} MB); this family is latency/FLOP-"
                       f"bound, not HBM-bound, so L2 residency does not affect the timing"),
     }
+
+
+DUMP_LIMIT = 64 << 20  # bytes written by --dump-outputs at most
+
+
+def dump_outputs(directory, outputs):
+    """Writes what one step() returned -- obs, reward, terminated, truncated and the info arrays ("info.<key>", nested keys
+    joined by ".") -- as <directory>/<name>.npy in float32 (flags, small integers) or float64 (other integers).  Above
+    DUMP_LIMIT bytes in all, every array keeps the same fixed, seeded sample of env rows, listed in env_index.npy."""
+    import numpy as np
+    import torch
+
+    obs, reward, terminated, truncated, info = outputs
+    arrays = {"obs": obs, "reward": reward, "terminated": terminated, "truncated": truncated}
+
+    def add_info(d, prefix):
+        for k, v in d.items():
+            if isinstance(v, dict):
+                add_info(v, f"{prefix}{k}.")
+            elif isinstance(v, torch.Tensor):
+                arrays[prefix + k] = v
+
+    add_info(info, "info.")
+    host = {}
+    for k, v in arrays.items():
+        a = v.detach().cpu().numpy()
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float32 if a.dtype.itemsize <= 2 else np.float64)
+        host[k] = a
+    n = len(host["reward"])
+    row_bytes = sum(a.nbytes for a in host.values()) / n
+    if row_bytes * n > DUMP_LIMIT:
+        m = int((DUMP_LIMIT - 1024 * len(host)) // (row_bytes + 8))  # 1 KB per file for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+        host = {k: a[idx] for k, a in host.items()}
+        host["env_index"] = idx.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
 
 
 def measure_e2e(cx, args, env_id, n, mode, tag):
@@ -765,7 +775,7 @@ def family_block(cx, args, env_id, n, K, W, with_sync_e2e, fma_cache, cpu_baseli
     """Everything measured for one family at this world size: device-timed value, roofline, pipelined e2e (+ NCCL variant)."""
     facts = ENV_FACTS[env_id]
     res = measure_device(cx, args, env_id, n, K, W, args.ring if env_id == args.env else 0)
-    envs, acts = res.pop("envs"), res.pop("acts")
+    envs, acts, outputs = res.pop("envs"), res.pop("acts"), res.pop("outputs")
     per_gpu = res["value"] / cx.world
     kernel_s = res["elapsed_s"] / res["timed_steps"]
     if env_id in FLOP_BOUND:
@@ -785,14 +795,13 @@ def family_block(cx, args, env_id, n, K, W, with_sync_e2e, fma_cache, cpu_baseli
                 "frac": achieved / cx.hbm_peak, "peak_source": cx.peak_src,
                 "algorithmic_bytes_per_env_step": facts["step_bytes"], "avg_launch_us": kernel_s * 1e6,
                 "traffic": load_ncu_traffic(facts["kernel"])}
-    block = {k: res[k] for k in ("value", "ms_per_step", "ms_per_step_p50", "ms_per_step_p95", "ms_per_step_min",
-                                 "timed_steps", "graph_launches", "replays", "reps_of_K", "l2_policy")}
+    block = {k: res[k] for k in ("value", "ms_per_step", "timed_steps", "graph_launches", "l2_policy")}
     block["timed_region_ms"] = res["elapsed_s"] * 1e3
     block["value_excluding_reset_calls"] = res["value"] * (1 - res["reset_frac"])
     block["reset_call_fraction"] = res["reset_frac"]
     block["roofline"] = roof
     block["gpu_launches"] = res["timed_steps"] * facts.get("launches_per_step", 1)
-    return block, envs, acts
+    return block, envs, acts, outputs
 
 
 def run_b200(args):
@@ -812,7 +821,10 @@ def run_b200(args):
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         cpu_baseline = cpu_baseline_subprocess(args, args.env, n, 12)
 
-    block, envs, acts = family_block(cx, args, args.env, n, K, W, True, fma_cache, cpu_baseline)
+    block, envs, acts, outputs = family_block(cx, args, args.env, n, K, W, True, fma_cache, cpu_baseline)
+    if args.dump_outputs and rank == 0:  # before anything else steps these batches
+        dump_outputs(args.dump_outputs, outputs)
+    del outputs
     extras = {}
     if not args.no_extras and rank == 0 and world == 1:  # supporting numbers belong to the 1-GPU line
         try:
@@ -835,7 +847,7 @@ def run_b200(args):
         hcpu = None
         if rank == 0 and world == 1 and not args.no_cpu_baseline:
             hcpu = cpu_baseline_subprocess(args, "Humanoid-v5", hn, 10)
-        humanoid, henvs, hacts = family_block(cx, args, "Humanoid-v5", hn, K, W, False, fma_cache, hcpu)
+        humanoid, henvs, hacts, _ = family_block(cx, args, "Humanoid-v5", hn, K, W, False, fma_cache, hcpu)
         del henvs, hacts
         torch.cuda.empty_cache()
         humanoid["e2e"] = measure_e2e(cx, args, "Humanoid-v5", hn, "dma", "hum")
@@ -866,14 +878,13 @@ def run_b200(args):
                             f"autoreset, TimeLimit, numpy-parity PCG64 streams",
                 "num_envs_per_gpu": n, "parallelism": f"env-shards x{world} (no data-path collective)",
                 "l2_policy": block["l2_policy"],
-                "launch": (f"one CUDA graph of {block['graph_launches']} step launches (= {block['graph_launches'] / K:g} x the "
-                           f"K={K} steps asked for) replayed {block['replays']} times: {block['timed_steps']} timed steps, "
-                           f"{block['timed_region_ms']:.1f} ms region, CUDA events on the launch stream around every replay"),
+                "launch": (f"one CUDA graph of {block['graph_launches']} step launches: {W} warm-up launches, then the "
+                           f"{block['timed_steps']} timed ones (--steps) between two CUDA event nodes of the graph, "
+                           f"{block['timed_region_ms']:.3f} ms region"),
                 "counting": "calls x N (reset calls included); see value_excluding_reset_calls",
                 "steady_state": (f"{BURN_IN[args.env]} untimed burn-in steps per batch before warm-up" if args.env in BURN_IN else None),
             },
-            "timing": {k: block[k] for k in ("timed_steps", "graph_launches", "replays", "reps_of_K", "timed_region_ms",
-                                             "ms_per_step_p50", "ms_per_step_p95", "ms_per_step_min")},
+            "timing": {k: block[k] for k in ("timed_steps", "graph_launches", "timed_region_ms")},
             "value_excluding_reset_calls": block["value_excluding_reset_calls"],
             "reset_call_fraction": block["reset_call_fraction"],
             "gpu_launches": block["gpu_launches"],
@@ -1101,7 +1112,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-humanoid", action="store_true", help="skip the Humanoid-v5 8192-envs/GPU block of the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of --env returned as DIR/<name>.npy (float32/float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

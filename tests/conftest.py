@@ -9,12 +9,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-# The host framework (Gymnasium) the engine plugs into: the offline install of the reference under baseline/_ref travels
-# with the repo snapshot.  It must be importable BEFORE gymnasium_b200 is first imported so the engine subclasses the
-# real gymnasium.vector.VectorEnv; B200ENV_FORCE_COMPAT=1 exercises the stand-in types instead.
-_REF = os.path.join(ROOT, "baseline", "_ref")
-if os.path.isdir(os.path.join(_REF, "gymnasium")) and _REF not in sys.path and not os.environ.get("B200ENV_FORCE_COMPAT"):
-    sys.path.insert(0, _REF)
 
 
 def pytest_configure(config):

@@ -186,9 +186,38 @@ def cartpole_beyond(name, n, T, seed):
     print(name, "term", term.sum(), "zero rewards", int((rew == 0).sum()))
 
 
+def dropin(name, env_id, n, T, seed, nA, spaces=False, **kw):
+    """The stock sync vectoriser's outputs and output dtypes on a seeded action tape, with its spaces if asked
+    (tests/test_gpu_dropin.py)."""
+    envs = gym.make_vec(env_id, num_envs=n, vectorization_mode="sync", **kw)
+    actions = np.random.default_rng(6000 + seed).integers(0, nA, size=(T, n)).astype(np.int64)
+    o, _ = envs.reset(seed=seed)
+    obs = [o]
+    rew, term, trunc = [], [], []
+    for t in range(T):
+        o, r, te, tr, _ = envs.step(actions[t])
+        obs.append(o); rew.append(r); term.append(te); trunc.append(tr)
+    out = dict(seed=np.int64(seed), actions=actions, obs=np.stack(obs), reward=np.stack(rew), terminated=np.stack(term),
+               truncated=np.stack(trunc), step_dtypes=np.array([str(r.dtype), str(te.dtype), str(tr.dtype)]))
+    for tag, sp in (("obs_space", envs.observation_space), ("single_obs_space", envs.single_observation_space),
+                    ("action_space", envs.action_space)) if spaces else ():
+        if isinstance(sp, gym.spaces.Box):
+            out.update({tag + "_low": sp.low, tag + "_high": sp.high})
+        else:
+            out.update({tag + "_nvec": sp.nvec, tag + "_start": sp.start})
+        out[tag + "_dtype"] = np.array(str(sp.dtype))
+    envs.close()
+    np.savez_compressed(os.path.join(HERE, name), **out)
+    print(name, {k: v.shape for k, v in out.items()}, "term", out["terminated"].sum(), "reward", out["reward"].sum())
+
+
 if __name__ == "__main__":
     assert "reference" in gym.__file__ or "_ref" in gym.__file__, gym.__file__
     print("reference:", gym.__version__, gym.__file__, "numpy", np.__version__)
+    if len(sys.argv) > 1 and sys.argv[1] == "dropin":  # regenerate only the drop-in fixtures
+        dropin("dropin_cartpole_n5_s123_T150.npz", "CartPole-v1", 5, 150, 123, 2, spaces=True)
+        dropin("dropin_frozenlake8x8_n6_s5_T200.npz", "FrozenLake-v1", 6, 200, 5, 4, map_name="8x8")
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "cartpole_beyond":
         cartpole_beyond("beyond_cartpole_n4_s5.npz", 4, 40, 5)
         sys.exit(0)

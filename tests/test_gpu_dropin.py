@@ -1,57 +1,75 @@
-"""Drop-in through Gymnasium's own registry (needs gymnasium importable: baseline/_ref travels with the snapshot)."""
+"""Drop-in through Gymnasium's own registry, checked against the stock sync vectoriser's spaces and outputs stored in
+tests/golden/dropin_*.npz (tests/golden/make_golden.py dropin).  Without Gymnasium installed, the same ids go through the
+engine's standalone make_vec (gymnasium_b200/registration.py) and are checked against the same fixtures."""
 import os
 import sys
 
 import numpy as np
 import pytest
 
-from conftest import ROOT, have_cuda
+from conftest import ROOT, golden, have_cuda
 
 pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not have_cuda(), reason="needs a CUDA device")]
 
-gym = pytest.importorskip("gymnasium")  # conftest.py puts baseline/_ref on sys.path when it exists
+
+def replay(env, g):
+    """Reset with the fixture's seed, step its action tape, and compare every output (and its dtype) with the fixture."""
+    np.testing.assert_array_equal(env.reset(seed=int(g["seed"]))[0], g["obs"][0])
+    for t, a in enumerate(g["actions"]):
+        x = env.step(a)
+        if x[0].dtype == np.float32:
+            np.testing.assert_allclose(x[0], g["obs"][t + 1], rtol=1e-5, atol=1e-5)
+        else:
+            np.testing.assert_array_equal(x[0], g["obs"][t + 1])
+        for k, name in ((1, "reward"), (2, "terminated"), (3, "truncated")):
+            np.testing.assert_array_equal(x[k], g[name][t])
+            assert str(x[k].dtype) == str(g["step_dtypes"][k - 1])
 
 
 def test_make_vec_through_the_registry():
     import gymnasium_b200
-    from gymnasium.vector import AutoresetMode, VectorEnv
 
-    assert gymnasium_b200.HAVE_GYMNASIUM
-    env = gym.make_vec("B200/CartPole-v1", num_envs=5, output="numpy")
-    assert isinstance(env, VectorEnv) and isinstance(env, gymnasium_b200.B200VectorEnv)
-    assert env.spec.id == "B200/CartPole-v1" and env.spec.kwargs["num_envs"] == 5
-    assert env.max_episode_steps == 500 and env.metadata["autoreset_mode"] is AutoresetMode.NEXT_STEP
-    ref = gym.make_vec("CartPole-v1", num_envs=5, vectorization_mode="sync")
-    assert env.observation_space == ref.observation_space and env.action_space == ref.action_space
-    assert env.single_observation_space == ref.single_observation_space
-    o1, _ = env.reset(seed=123)
-    o2, _ = ref.reset(seed=123)
-    np.testing.assert_array_equal(o1, o2)
-    rs = np.random.default_rng(0)
-    for _ in range(150):
-        a = ref.action_space.sample()
-        x, y = env.step(a), ref.step(a)
-        np.testing.assert_allclose(x[0], y[0], rtol=1e-5, atol=1e-5)
-        for k in (1, 2, 3):
-            np.testing.assert_array_equal(x[k], y[k])
-            assert x[k].dtype == y[k].dtype
-    env.close(); ref.close()
+    g = golden("dropin_cartpole_n5_s123_T150.npz")
+    if gymnasium_b200.HAVE_GYMNASIUM:
+        import gymnasium as gym
+        from gymnasium.vector import VectorEnv
+
+        env = gym.make_vec("B200/CartPole-v1", num_envs=5, output="numpy")
+        assert isinstance(env, VectorEnv)
+        assert env.spec.id == "B200/CartPole-v1" and env.spec.kwargs["num_envs"] == 5
+    else:
+        env = gymnasium_b200.make_vec("B200/CartPole-v1", num_envs=5, output="numpy")
+    assert isinstance(env, gymnasium_b200.B200VectorEnv)
+    assert env.max_episode_steps == 500 and env.metadata["autoreset_mode"] is gymnasium_b200.AutoresetMode.NEXT_STEP
+    for tag, sp in (("obs_space", env.observation_space), ("single_obs_space", env.single_observation_space)):
+        # Box equality as gymnasium.spaces.Box.__eq__ defines it: shape, dtype, np.allclose bounds
+        assert str(sp.dtype) == str(g[tag + "_dtype"]) and sp.shape == g[tag + "_low"].shape
+        assert np.allclose(sp.low, g[tag + "_low"]) and np.allclose(sp.high, g[tag + "_high"])
+    assert str(env.action_space.dtype) == str(g["action_space_dtype"])
+    np.testing.assert_array_equal(env.action_space.nvec, g["action_space_nvec"])
+    np.testing.assert_array_equal(env.action_space.start, g["action_space_start"])
+    replay(env, g)
+    env.close()
 
 
 def test_install_routes_stock_ids():
     import gymnasium_b200
 
+    g = golden("dropin_frozenlake8x8_n6_s5_T200.npz")
+    if not gymnasium_b200.HAVE_GYMNASIUM:
+        with pytest.raises(RuntimeError, match="gymnasium is not importable"):
+            gymnasium_b200.install(["FrozenLake-v1"])
+        env = gymnasium_b200.make_vec("FrozenLake-v1", num_envs=6, map_name="8x8", output="numpy")
+        assert env.max_episode_steps == 100
+        replay(env, g)
+        return
+    import gymnasium as gym
+
     gymnasium_b200.install(["FrozenLake-v1"])
     try:
         env = gym.make_vec("FrozenLake-v1", num_envs=6, map_name="8x8", output="numpy")
         assert isinstance(env, gymnasium_b200.B200VectorEnv) and env.max_episode_steps == 100
-        ref = gym.make_vec("FrozenLake-v1", num_envs=6, map_name="8x8", vectorization_mode="sync")
-        np.testing.assert_array_equal(env.reset(seed=5)[0], ref.reset(seed=5)[0])
-        for _ in range(200):
-            a = ref.action_space.sample()
-            x, y = env.step(a), ref.step(a)
-            for k in range(4):
-                np.testing.assert_array_equal(x[k], y[k])
+        replay(env, g)
     finally:
         gymnasium_b200.uninstall()
 

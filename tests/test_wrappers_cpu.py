@@ -1,13 +1,21 @@
 """On-device vector wrappers (gymnasium_b200/wrappers.py) against the reference's NumPy wrappers, driven by the same
-scripted vector env (CPU tensors: the wrappers are device-agnostic torch code)."""
+scripted vector env (CPU tensors: the wrappers are device-agnostic torch code).  The reference's outputs on these tapes
+are stored in tests/golden/wrappers_reference.npz (tests/golden/make_golden_wrappers.py)."""
+import functools
+
 import numpy as np
 import pytest
 import torch
 
-gym = pytest.importorskip("gymnasium")
-from gymnasium.vector import AutoresetMode, VectorEnv  # noqa: E402
+from conftest import golden
 
-from gymnasium_b200 import wrappers as W  # noqa: E402
+from gymnasium_b200 import wrappers as W
+from gymnasium_b200._api import AutoresetMode, Box, Discrete, VectorEnv, batch_space
+
+
+@functools.cache
+def reference():
+    return golden("wrappers_reference.npz")
 
 
 class ScriptedEnv(VectorEnv):
@@ -17,10 +25,10 @@ class ScriptedEnv(VectorEnv):
         rs = np.random.default_rng(seed)
         self.num_envs = n
         self.metadata = {"autoreset_mode": mode}
-        self.single_observation_space = gym.spaces.Box(-np.inf, np.inf, (3,), np.float32)
-        self.single_action_space = gym.spaces.Discrete(2)
-        self.observation_space = gym.vector.utils.batch_space(self.single_observation_space, n)
-        self.action_space = gym.vector.utils.batch_space(self.single_action_space, n)
+        self.single_observation_space = Box(-np.inf, np.inf, (3,), np.float32)
+        self.single_action_space = Discrete(2)
+        self.observation_space = batch_space(self.single_observation_space, n)
+        self.action_space = batch_space(self.single_action_space, n)
         self.obs = rs.normal(1.5, 2.0, size=(T + 1, n, 3)).astype(np.float32)
         self.rew = rs.normal(0.3, 1.0, size=(T, n))
         self.term = rs.random((T, n)) < 0.07
@@ -49,60 +57,54 @@ class ScriptedEnv(VectorEnv):
 
 @pytest.mark.parametrize("mode", [AutoresetMode.NEXT_STEP, AutoresetMode.SAME_STEP])
 def test_record_episode_statistics_matches_reference(mode):
-    from gymnasium.wrappers.vector import RecordEpisodeStatistics as Ref
-
+    REF, p = reference(), f"res_{mode.name.lower()}_"
     n, T = 6, 120
-    ref = Ref(ScriptedEnv(n, T, 1, False, mode), buffer_length=50)
     mine = W.RecordEpisodeStatistics(ScriptedEnv(n, T, 1, True, mode), buffer_length=50)
-    ref.reset(); mine.reset()
+    mine.reset()
     for t in range(T):
         a = np.zeros(n, dtype=np.int64)
-        _, _, te, tr, ri = ref.step(a)
         _, _, te2, tr2, mi = mine.step(a)
-        done = te | tr
+        done = REF[p + "done"][t]
         np.testing.assert_array_equal(mi["_episode"].numpy(), done)
         if done.any():
-            np.testing.assert_allclose(mi["episode"]["r"].numpy(), ri["episode"]["r"], rtol=0, atol=1e-12)
-            np.testing.assert_array_equal(mi["episode"]["l"].numpy(), ri["episode"]["l"])
-            np.testing.assert_array_equal(ri["_episode"], done)
+            assert REF[p + "ep_present"][t]
+            np.testing.assert_allclose(mi["episode"]["r"].numpy(), REF[p + "ep_r"][t], rtol=0, atol=1e-12)
+            np.testing.assert_array_equal(mi["episode"]["l"].numpy(), REF[p + "ep_l"][t])
+            np.testing.assert_array_equal(REF[p + "ep_mask"][t], done)
         else:
-            assert "episode" not in ri and float(mi["episode"]["r"].abs().sum()) == 0.0
-    assert mine.episode_count == ref.episode_count
-    np.testing.assert_allclose(np.sort(mine.return_queue.numpy()), np.sort(np.array(ref.return_queue)), atol=1e-12)
-    np.testing.assert_array_equal(np.sort(mine.length_queue.numpy()), np.sort(np.array(ref.length_queue)))
+            assert not REF[p + "ep_present"][t] and float(mi["episode"]["r"].abs().sum()) == 0.0
+    assert mine.episode_count == int(REF[p + "episode_count"])
+    np.testing.assert_allclose(np.sort(mine.return_queue.numpy()), np.sort(REF[p + "return_queue"]), atol=1e-12)
+    np.testing.assert_array_equal(np.sort(mine.length_queue.numpy()), np.sort(REF[p + "length_queue"]))
     # a buffer smaller than the number of episodes (and than the finishers of one step): same entries, same (chronological)
     # order as the reference's deques
-    ref = Ref(ScriptedEnv(n, T, 1, False, mode), buffer_length=4)
     mine = W.RecordEpisodeStatistics(ScriptedEnv(n, T, 1, True, mode), buffer_length=4)
-    ref.reset(); mine.reset()
+    mine.reset()
     for t in range(T):
-        ref.step(np.zeros(n, dtype=np.int64)); mine.step(np.zeros(n, dtype=np.int64))
-        np.testing.assert_allclose(mine.return_queue.numpy(), np.array(ref.return_queue), atol=1e-12, err_msg=f"step {t}")
-        np.testing.assert_array_equal(mine.length_queue.numpy(), np.array(ref.length_queue))
+        mine.step(np.zeros(n, dtype=np.int64))
+        k = int(REF[p + "q4_len"][t])
+        np.testing.assert_allclose(mine.return_queue.numpy(), REF[p + "rq4"][t, :k], atol=1e-12, err_msg=f"step {t}")
+        np.testing.assert_array_equal(mine.length_queue.numpy(), REF[p + "lq4"][t, :k])
 
 
 def test_normalize_observation_and_reward_match_reference():
-    from gymnasium.wrappers.vector import NormalizeObservation as RefO
-    from gymnasium.wrappers.vector import NormalizeReward as RefR
-
+    REF = reference()
     n, T = 8, 90
-    ro, mo = RefO(ScriptedEnv(n, T, 2, False)), W.NormalizeObservation(ScriptedEnv(n, T, 2, True))
-    rr, mr = RefR(ScriptedEnv(n, T, 3, False), gamma=0.97), W.NormalizeReward(ScriptedEnv(n, T, 3, True), gamma=0.97)
-    o1, _ = ro.reset(); o2, _ = mo.reset()
-    np.testing.assert_allclose(o2.numpy(), o1, rtol=1e-4, atol=1e-5)
-    rr.reset(); mr.reset()
+    mo = W.NormalizeObservation(ScriptedEnv(n, T, 2, True))
+    mr = W.NormalizeReward(ScriptedEnv(n, T, 3, True), gamma=0.97)
+    o2, _ = mo.reset()
+    np.testing.assert_allclose(o2.numpy(), REF["no_obs"][0], rtol=1e-4, atol=1e-5)
+    mr.reset()
     for t in range(T):
         a = np.zeros(n, dtype=np.int64)
-        o1, *_ = ro.step(a)
         o2, *_ = mo.step(a)
         assert o2.dtype == torch.float32
-        np.testing.assert_allclose(o2.numpy(), o1, rtol=1e-4, atol=1e-5)
-        _, r1, *_ = rr.step(a)
+        np.testing.assert_allclose(o2.numpy(), REF["no_obs"][t + 1], rtol=1e-4, atol=1e-5)
         _, r2, *_ = mr.step(a)
         # the reference takes np.mean/np.var of a float32 array (float32 pairwise sums); ours reduces in float64
-        np.testing.assert_allclose(r2.numpy(), r1, rtol=2e-6, atol=1e-9)
-    np.testing.assert_allclose(mo.obs_rms.mean.numpy(), ro.obs_rms.mean, rtol=1e-4, atol=1e-5)
-    np.testing.assert_allclose(float(mr.return_rms.var), float(rr.return_rms.var), rtol=2e-6)
+        np.testing.assert_allclose(r2.numpy(), REF["nr_rew"][t], rtol=2e-6, atol=1e-9)
+    np.testing.assert_allclose(mo.obs_rms.mean.numpy(), REF["no_mean"], rtol=1e-4, atol=1e-5)
+    np.testing.assert_allclose(float(mr.return_rms.var), float(REF["nr_var"]), rtol=2e-6)
     with pytest.raises(ValueError):
         W.NormalizeObservation(ScriptedEnv(2, 3, 0, True), epsilon=0)
     with pytest.raises(ValueError):
@@ -132,14 +134,36 @@ class InfoEnv(ScriptedEnv):
         return out[:4] + (self._info(self.t),)
 
 
-def test_dict_info_to_list_matches_reference():
-    from gymnasium.wrappers.vector import DictInfoToList as Ref
+def reference_info_list(t):
+    """The reference DictInfoToList's list of per-env dicts at call t, rebuilt from the stored presence masks and values
+    (an entry "a.b" is key b of the nested dict under key a)."""
+    REF = reference()
+    paths =[str(s) for s in REF["dil_paths"]]
+    out = []
+    for i in range(REF["dil_present_" + paths[0]].shape[1]):
+        d = {}
+        for path in paths:
+            if not REF["dil_present_" + path][t, i]:
+                continue
+            *parents, key = path.split(".")
+            node = d
+            for q in parents:
+                node = node.setdefault(q, {})
+            if "dil_value_" + path in REF:
+                node[key] = REF["dil_value_" + path][t, i]
+            else:
+                node.setdefault(key, {})
+        out.append(d)
+    return out
 
+
+def test_dict_info_to_list_matches_reference():
     n, T = 6, 12
-    ref, ours = Ref(InfoEnv(n, T, 3, False)), W.DictInfoToList(InfoEnv(n, T, 3, True))
-    (_, ia), (_, ib) = ref.reset(seed=0), ours.reset(seed=0)
+    ours = W.DictInfoToList(InfoEnv(n, T, 3, True))
+    _, ib = ours.reset(seed=0)
     for t in range(T + 1):
-        assert isinstance(ib, list) and len(ib) == n
+        ia = reference_info_list(t)
+        assert isinstance(ib, list) and len(ib) == n == len(ia)
         for a, b in zip(ia, ib):
             assert set(a) == set(b)
             for k in a:
@@ -150,7 +174,7 @@ def test_dict_info_to_list_matches_reference():
                 else:
                     assert a[k] == b[k] and np.asarray(b[k]).dtype == np.asarray(a[k]).dtype
         if t < T:
-            ia, ib = ref.step(np.zeros(n, dtype=np.int64))[4], ours.step(np.zeros(n, dtype=np.int64))[4]
+            ib = ours.step(np.zeros(n, dtype=np.int64))[4]
 
 
 def test_numpy_to_torch_outputs_are_the_numpy_env_outputs_as_tensors():
