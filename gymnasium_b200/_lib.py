@@ -9,7 +9,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# B2E_LIB_PATH: load another build of the same library (A/B measurements of kernel variants, scripts/lanes_sweep.py)
+# B2E_LIB_PATH: load another build of the same library (e.g. one installed elsewhere, or a build to compare against)
 LIB_PATH = os.environ.get("B2E_LIB_PATH") or os.path.join(_HERE, "libb200env.so")
 
 # enums (include/b200env.h)
@@ -38,7 +38,7 @@ class Batch(C.Structure):
 class CartPoleCfg(C.Structure):
     """``b2e_cartpole_cfg``."""
 
-    _fields_ = [("reset_low", c_double), ("reset_high", c_double), ("sutton_barto_reward", c_i32), ("step_block", c_i32)]
+    _fields_ = [("reset_low", c_double), ("reset_high", c_double), ("sutton_barto_reward", c_i32)]
 
 
 class FrozenLakeCfg(C.Structure):
@@ -72,15 +72,15 @@ class BlackjackCfg(C.Structure):
 class LunarLanderCfg(C.Structure):
     """``b2e_lunarlander_cfg``."""
 
-    _fields_ = [("gravity", c_double), ("enable_wind", c_i32), ("continuous", c_i32), ("lanes_per_warp", c_i32),
-                ("grouping", c_i32), ("wind_power", c_double), ("turbulence_power", c_double)]
+    _fields_ = [("gravity", c_double), ("enable_wind", c_i32), ("continuous", c_i32), ("wind_power", c_double),
+                ("turbulence_power", c_double)]
 
 
 class LunarLanderState(C.Structure):
     """``b2e_lunarlander_state`` (device pointers)."""
 
     _fields_ = [(k, c_void_p) for k in ("bodies", "joints", "terrain", "fat", "contacts", "flags", "prev_shaping",
-                                        "ctrl", "rng", "work", "order", "wind", "u32buf")]
+                                        "ctrl", "rng", "wind", "u32buf")]
 
 
 class HumanoidCfg(C.Structure):
@@ -89,8 +89,7 @@ class HumanoidCfg(C.Structure):
     _fields_ = [(k, c_double) for k in ("reset_noise_scale", "forward_reward_weight", "ctrl_cost_weight",
                                         "contact_cost_weight", "contact_cost_max", "healthy_reward", "healthy_z_min",
                                         "healthy_z_max")] + [("terminate_when_unhealthy", c_i32), ("frame_skip", c_i32),
-                                                             ("lanes_per_warp", c_i32), ("impl", c_i32),
-                                                             ("envs_per_cta", c_i32), ("schedule", c_i32)]
+                                                             ("impl", c_i32), ("_pad", c_i32)]
 
 
 class HumanoidState(C.Structure):
@@ -106,7 +105,7 @@ class MjPlanarCfg(C.Structure):
     _fields_ = [(k, c_double) for k in ("reset_noise_scale", "forward_reward_weight", "ctrl_cost_weight", "healthy_reward",
                                         "healthy_z_min", "healthy_z_max", "healthy_angle_min", "healthy_angle_max",
                                         "healthy_state_min", "healthy_state_max")] + [
-        ("terminate_when_unhealthy", c_i32), ("frame_skip", c_i32), ("lanes_per_warp", c_i32), ("_pad", c_i32)]
+        ("terminate_when_unhealthy", c_i32), ("frame_skip", c_i32)]
 
 
 class MjPlanarState(C.Structure):
@@ -134,7 +133,7 @@ class PipeSlot(C.Structure):
     _fields_ = [("staging_host", c_void_p), ("actions_dev", c_void_p), ("action_bytes", C.c_size_t),
                 ("calls", C.POINTER(Call)), ("segs", C.POINTER(CopySeg)), ("ncalls", c_i32), ("nsegs", c_i32),
                 ("ev_h2d", c_void_p), ("ev_step", c_void_p), ("ev_copy", c_void_p), ("h2d_pending", c_i32),
-                ("copy_pending", c_i32), ("seq_src", c_void_p), ("copy_graph", c_void_p), ("land", c_void_p)]
+                ("copy_pending", c_i32), ("land", c_void_p)]
 
 
 P = c_void_p
@@ -151,12 +150,11 @@ SIGNATURES = {
     "b2e_copy_to_host_async": (C.c_int, [P, c_i32, P]),
     "b2e_pipe_slot_init": (C.c_int, [C.POINTER(PipeSlot)]),
     "b2e_pipe_slot_destroy": (C.c_int, [C.POINTER(PipeSlot)]),
-    "b2e_pipe_slot_capture": (C.c_int, [C.POINTER(PipeSlot), P]),
     "b2e_pipe_slot_land_kernel": (C.c_int, [C.POINTER(PipeSlot)]),
     "b2e_land_plan_create": (C.c_int, [P, c_i32, P, C.POINTER(c_void_p)]),
     "b2e_land_plan_launch": (C.c_int, [P, c_i64, P]),
     "b2e_land_plan_destroy": (C.c_int, [P]),
-    "b2e_pipe_submit": (C.c_int, [C.POINTER(PipeSlot), P, P, P, P, c_i64, P, c_i64, c_i32, c_double]),
+    "b2e_pipe_submit": (C.c_int, [C.POINTER(PipeSlot), P, P, P, P, c_i64, c_i64, c_i32, c_double]),
     "b2e_rng_seed": (C.c_int, [_BP, c_u64, P, P, P, P]),
     "b2e_rng_random": (C.c_int, [_BP, P, c_i32, P, P]),
     "b2e_cartpole_reset": (C.c_int, [_BP, C.POINTER(CartPoleCfg), P, P, P, P, P, P]),

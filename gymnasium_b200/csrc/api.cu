@@ -258,7 +258,6 @@ extern "C" int b2e_pipe_slot_init(b2e_pipe_slot* s) {
   s->ev_step = ev[1];
   s->ev_copy = ev[2];
   s->h2d_pending = s->copy_pending = 0;
-  s->copy_graph = nullptr;
   s->land = nullptr;
   return 0;
 }
@@ -310,9 +309,7 @@ extern "C" int b2e_land_plan_create(const b2e_copy_seg* segs, int32_t count, int
   cudaGetDevice(&dev_id);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev_id);
   // few CTAs: measured on B200 (scripts/link_probe.py, 1.7 MB): 37 CTAs 40.9 us, 148 CTAs 41.9, 296+ CTAs 45.8 (copy engine: 33.3)
-  size_t cap = (size_t)(sms / 4 > 0 ? sms / 4 : 1);
-  if (const char* e = getenv("B2E_LAND_GRID"))
-    if (atoi(e) > 0) cap = (size_t)atoi(e);
+  const size_t cap = (size_t)(sms / 4 > 0 ? sms / 4 : 1);
   const size_t want = (chunks + 255) / 256;
   p->grid = (int)(want < 1 ? 1 : (want > cap ? cap : want));
   *plan_out = p;
@@ -348,35 +345,6 @@ extern "C" int b2e_pipe_slot_land_kernel(b2e_pipe_slot* s) {
   return b2e_land_plan_create(s->segs, s->nsegs - 2, (int64_t*)s->segs[s->nsegs - 1].host_dst, &s->land);
 }
 
-extern "C" int b2e_pipe_slot_capture(b2e_pipe_slot* s, void* copy_stream) {
-  if (!s || !s->segs || s->nsegs < 2 || !s->seq_src) {
-    set_error("b2e_pipe_slot_capture: slot, segments or seq_src missing");
-    return B2E_EINVAL;
-  }
-  if (s->copy_graph) return 0;
-  cudaStream_t cs = (cudaStream_t)copy_stream;
-  s->segs[s->nsegs - 2].dev_src = s->seq_src;  // the sequence word always travels from the slot's own page-locked word
-  if (int st = cuda_status(cudaStreamBeginCapture(cs, cudaStreamCaptureModeRelaxed), "b2e_pipe_slot_capture (begin)")) return st;
-  const int st_copy = b2e_copy_to_host_async(s->segs, s->nsegs, copy_stream);
-  cudaGraph_t graph = nullptr;
-  const cudaError_t e_end = cudaStreamEndCapture(cs, &graph);
-  if (st_copy) {
-    if (graph) cudaGraphDestroy(graph);
-    return st_copy;
-  }
-  if (int st = cuda_status(e_end, "b2e_pipe_slot_capture (end)")) return st;
-  cudaGraphExec_t exec = nullptr;
-  const cudaError_t e_inst = cudaGraphInstantiate(&exec, graph, 0);
-  cudaGraphDestroy(graph);
-  if (int st = cuda_status(e_inst, "b2e_pipe_slot_capture (instantiate)")) return st;
-  if (int st = cuda_status(cudaGraphUpload(exec, cs), "b2e_pipe_slot_capture (upload)")) {
-    cudaGraphExecDestroy(exec);
-    return st;
-  }
-  s->copy_graph = exec;
-  return 0;
-}
-
 extern "C" int b2e_pipe_slot_destroy(b2e_pipe_slot* s) {
   if (!s) return 0;
   void** ev[3] = {&s->ev_h2d, &s->ev_step, &s->ev_copy};
@@ -385,10 +353,6 @@ extern "C" int b2e_pipe_slot_destroy(b2e_pipe_slot* s) {
       cudaEventDestroy((cudaEvent_t)*ev[i]);
       *ev[i] = nullptr;
     }
-  if (s->copy_graph) {
-    cudaGraphExecDestroy((cudaGraphExec_t)s->copy_graph);
-    s->copy_graph = nullptr;
-  }
   if (s->land) {
     b2e_land_plan_destroy(s->land);
     s->land = nullptr;
@@ -400,16 +364,14 @@ typedef int (*b2e_anyfn)(uint64_t, uint64_t, uint64_t, uint64_t, uint64_t, uint6
                          uint64_t, uint64_t, uint64_t, uint64_t, uint64_t, uint64_t);
 
 extern "C" int b2e_pipe_submit(b2e_pipe_slot* s, const void* host_actions, void* main_stream, void* copy_stream,
-                               const int64_t* ack_word, int64_t need_ack, void* seq_src, int64_t seq_value, int32_t flags,
-                               double timeout_s) {
-  if (!s || !host_actions || !s->actions_dev || !s->calls || !s->segs || s->nsegs < 2) {
+                               const int64_t* ack_word, int64_t need_ack, int64_t seq_value, int32_t flags, double timeout_s) {
+  if (!s || !host_actions || !s->actions_dev || !s->calls) {
     set_error("b2e_pipe_submit: null pointer in the slot or its arguments");
     return B2E_EINVAL;
   }
-  int64_t* const seq_word = s->land ? (int64_t*)s->segs[s->nsegs - 1].host_dst : s->copy_graph ? s->seq_src : (int64_t*)seq_src;
   const bool pinned = (flags & B2E_PIPE_ACTIONS_PINNED) != 0;
-  if (!seq_word || (!pinned && !s->staging_host)) {
-    set_error("b2e_pipe_submit: no sequence-word source, or no staging buffer for pageable actions");
+  if (!s->land || (!pinned && !s->staging_host)) {
+    set_error("b2e_pipe_submit: no landing kernel (b2e_pipe_slot_land_kernel), or no staging buffer for pageable actions");
     return B2E_EINVAL;
   }
   cudaStream_t ms = (cudaStream_t)main_stream, cs = (cudaStream_t)copy_stream;
@@ -465,23 +427,9 @@ extern "C" int b2e_pipe_submit(b2e_pipe_slot* s, const void* host_actions, void*
       }
     }
   }
-  // (5) land the outputs + the sequence word.  Its page-locked source is written only now: once the slot has been released,
-  // the copy that published the slot's previous step has certainly read it.
-  if (s->land) {  // the SMs store the rows and then the word itself
-    if (int st = b2e_land_plan_launch(s->land, seq_value, copy_stream)) return st;
-    cudaEventRecord((cudaEvent_t)s->ev_copy, cs);
-    s->copy_pending = 1;
-    return cuda_status(cudaGetLastError(), "b2e_pipe_submit (landing kernel)");
-  }
-  *(volatile int64_t*)seq_word = seq_value;
-  __atomic_thread_fence(__ATOMIC_RELEASE);
-  if (s->copy_graph) {
-    if (int st = cuda_status(cudaGraphLaunch((cudaGraphExec_t)s->copy_graph, cs), "b2e_pipe_submit (landing graph)")) return st;
-  } else {
-    s->segs[s->nsegs - 2].dev_src = seq_word;
-    if (int st = b2e_copy_to_host_async(s->segs, s->nsegs, copy_stream)) return st;
-  }
+  // (5) the SMs store the outputs into the host batch, then the sequence word
+  if (int st = b2e_land_plan_launch(s->land, seq_value, copy_stream)) return st;
   cudaEventRecord((cudaEvent_t)s->ev_copy, cs);
   s->copy_pending = 1;
-  return cuda_status(cudaGetLastError(), "b2e_pipe_submit");
+  return cuda_status(cudaGetLastError(), "b2e_pipe_submit (landing kernel)");
 }

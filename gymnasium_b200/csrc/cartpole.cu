@@ -13,8 +13,8 @@
 // Memory: struct-of-arrays float64 state [4][n] (four fully coalesced 8-byte streams), one packed int32 control word,
 // float4 observation store, RNG state touched only by lanes that reset.  HBM-bound: 106 B/env-step with int64 actions.
 // Round 2 tried two 16-byte state streams (LDG.128) and moving the rare code (autoreset draws, libdevice sincos) out of
-// line; a same-box A/B of the four combinations (scripts/cartpole_ab.sh, profiles/r2_notes.md) put this form first on the
-// HBM-cold ring (3.98 us per 65536-env launch against 4.03 / 4.04 / 4.11), so it is the default and the others are build knobs.
+// line; a same-box A/B of the four combinations (profiles/r2_notes.md) put this form first on the HBM-cold ring (3.98 us
+// per 65536-env launch against 4.03 / 4.04 / 4.11), so it is the only one kept.
 #include "common.cuh"
 
 namespace b2e {
@@ -56,14 +56,8 @@ __device__ __forceinline__ double div_total_mass(double x) {
   return __fma_rn(__fma_rn(-q, d, x), r, q);
 }
 
-// A/B knobs (scripts/cartpole_ab.sh builds the variants; profiles/r2_notes.md has the same-box measurement that picked the
-// defaults): state layout -- four 8-byte streams [4][n] (default) or two 16-byte streams (-DB2E_CARTPOLE_AB_AOS2); the
-// autoreset / libdevice-sincos code inlined (default) or out of line (-DB2E_CARTPOLE_AB_COLD=__noinline__).
-#ifndef B2E_CARTPOLE_AB_COLD
-#define B2E_CARTPOLE_AB_COLD __forceinline__
-#endif
-// libdevice's sincos (Payne-Hanek reduction and all), out of line and returning in registers
-__device__ B2E_CARTPOLE_AB_COLD double2 sincos_cold(double x) {
+// libdevice's sincos (Payne-Hanek reduction and all), returning in registers
+__device__ __forceinline__ double2 sincos_cold(double x) {
   double sn, cs;
   sincos(x, &sn, &cs);
   return make_double2(sn, cs);
@@ -124,23 +118,13 @@ __device__ __forceinline__ bool is_terminated(const State4& s) {  // cartpole.py
 }
 
 __device__ __forceinline__ State4 load_state(const double* __restrict__ st, int64_t n, int64_t i) {
-#ifdef B2E_CARTPOLE_AB_AOS2  // A/B builds only
-  const double2 a = reinterpret_cast<const double2*>(st)[i], b = reinterpret_cast<const double2*>(st)[n + i];
-  return State4{a.x, a.y, b.x, b.y};
-#else
   return State4{st[i], st[n + i], st[2 * n + i], st[3 * n + i]};
-#endif
 }
 __device__ __forceinline__ void store_state(double* __restrict__ st, int64_t n, int64_t i, const State4& s) {
-#ifdef B2E_CARTPOLE_AB_AOS2
-  reinterpret_cast<double2*>(st)[i] = make_double2(s.x, s.xd);
-  reinterpret_cast<double2*>(st)[n + i] = make_double2(s.th, s.thd);
-#else
   st[i] = s.x;
   st[n + i] = s.xd;
   st[2 * n + i] = s.th;
   st[3 * n + i] = s.thd;
-#endif
 }
 __device__ __forceinline__ float4 to_obs(const State4& s) {
   return make_float4((float)s.x, (float)s.xd, (float)s.th, (float)s.thd);
@@ -169,7 +153,6 @@ __device__ __forceinline__ State4 sample_reset(const A& a, int64_t i, uint64_t c
 }
 
 __global__ void __launch_bounds__(kBlock) cartpole_reset_kernel(const CartPoleArgs a) {
-  pdl_prologue();
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
   if (a.mask != nullptr && a.mask[i] == 0) return;
@@ -179,23 +162,14 @@ __global__ void __launch_bounds__(kBlock) cartpole_reset_kernel(const CartPoleAr
   reinterpret_cast<float4*>(a.obs)[i] = to_obs(s);
 }
 
-// The autoreset path of the step kernel, out of line (see the file header): CartPoleEnv.reset for one env -- draws, state,
-// cleared control word, observation.  Scalar arguments only, so that the call costs the hot path nothing (a reference to
-// the kernel's argument struct would make ptxas copy all of it to local memory in the kernel prologue).  `g` carries the
-// env's PCG64 words when the caller has already loaded them (numpy mode, kSpecRng).
-__device__ B2E_CARTPOLE_AB_COLD void reset_env_cold(double* __restrict__ state, int32_t* __restrict__ ctrl, uint64_t* __restrict__ rng,
-                                            float* __restrict__ obs, int64_t n, int64_t i, double low, double range,
-                                            int32_t rng_mode, uint64_t philox_seed, uint64_t env, uint64_t counter,
-                                            bool have_words, ulonglong2 w_state, ulonglong2 w_inc) {
+// The autoreset path of the step kernel: CartPoleEnv.reset for one env -- draws, state, cleared control word,
+// observation.  The PCG64 words are loaded here, by the resetting lanes only.
+__device__ __forceinline__ void reset_env_cold(double* __restrict__ state, int32_t* __restrict__ ctrl, uint64_t* __restrict__ rng,
+                                               float* __restrict__ obs, int64_t n, int64_t i, double low, double range,
+                                               int32_t rng_mode, uint64_t philox_seed, uint64_t env, uint64_t counter) {
   State4 s;
   if (rng_mode == B2E_RNG_NUMPY) {
-    Pcg64 g;
-    if (have_words) {
-      g.state = u128{w_state.x, w_state.y};
-      g.inc = u128{w_inc.x, w_inc.y};
-    } else {
-      g = pcg64_load(rng, n, i);
-    }
+    Pcg64 g = pcg64_load(rng, n, i);
     s.x = g.uniform(low, range);  // cartpole.py:236-241: x, x_dot, theta, theta_dot in this order
     s.xd = g.uniform(low, range);
     s.th = g.uniform(low, range);
@@ -213,36 +187,27 @@ __device__ B2E_CARTPOLE_AB_COLD void reset_env_cold(double* __restrict__ state, 
   __stcs(reinterpret_cast<float4*>(obs) + i, to_obs(s));
 }
 
-// One thread per env.  All loads are issued before the first use (one memory round trip).  kSpecRng: the PCG64 words of
-// EVERY lane are loaded up front together with the state (+32 B/env of reads, ~5 % of the lanes need them) -- with ~5 % of
-// the lanes on an autoreset call, 4 warps out of 5 contain one, and a load that depends on the control word would put a
-// second memory round trip on the critical path of a launch that lasts 3 us.  Opt-in (B2E_CARTPOLE_SPEC_RNG=1, batches up
-// to 2^21 envs): it pays off only while the batch is L2-resident, see launch_step.
+// One thread per env.  State, control word and action are issued before the first use (one memory round trip); the
+// PCG64 words are read only by the lanes that reset.  Loading them up front for every lane was measured on a B200 at
+// N=65536 (profiles/r2_notes.md): 3.03 vs 3.13 us per launch while the batch is L2-resident, but 3.84 vs 3.66 us on the
+// HBM-cold ring, where the +30 % DRAM reads outweigh the saved round trip.
 // Launch geometry was swept on a B200 at N=65536 (graph-chained launches, us per launch, L2-resident / HBM-cold ring):
 // CTA 64: 3.01 / 3.91, 128: 3.21 / 4.05, 256: 3.33 / 4.08, 448 (one CTA per SM): 3.28 / 4.01, 1024: 4.65 / 5.29; 2 or 4
 // envs per thread were slower (4.10 / 6.3 us L2-resident); programmatic dependent launch made N >= 65536 slower (4.07 vs
-// 3.27 us) and is opt-in (B2E_PDL=1).  b2e_cartpole_cfg.step_block overrides the CTA size.
+// 3.27 us).
 constexpr int kStepBlock = 64;
-constexpr int64_t kSpecRngMaxEnvs = 1 << 21;
 
-template <typename ActT, bool kSpecRng>
+template <typename ActT>
 __global__ void __launch_bounds__(1024) cartpole_step_kernel(const CartPoleArgs a) {
-  pdl_prologue();
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
   const int32_t c = a.ctrl[i];
   const State4 s0 = load_state(a.state, a.n, i);
   const int action = load_action<ActT>(a.actions, i);
-  ulonglong2 w_state = make_ulonglong2(0, 0), w_inc = make_ulonglong2(0, 0);
-  const bool have_words = kSpecRng && a.rng_mode == B2E_RNG_NUMPY;
-  if (have_words) {
-    w_state = reinterpret_cast<const ulonglong2*>(a.rng)[i];
-    w_inc = __ldg(reinterpret_cast<const ulonglong2*>(a.rng) + a.n + i);
-  }
   if (a.mode == B2E_AUTORESET_NEXT_STEP && ctrl_pending(c)) {
     // sync_vector_env.py:279-284: the call after a done is the reset; reward 0, flags False, action ignored
     reset_env_cold(a.state, a.ctrl, a.rng, a.obs, a.n, i, a.low, a.range, a.rng_mode, a.philox_seed,
-                   (uint64_t)(a.env_offset + i), a.call_counter, have_words, w_state, w_inc);
+                   (uint64_t)(a.env_offset + i), a.call_counter);
     __stcs(a.reward + i, 0.0);
     a.term[i] = 0;
     a.trunc[i] = 0;
@@ -265,7 +230,7 @@ __global__ void __launch_bounds__(1024) cartpole_step_kernel(const CartPoleArgs 
     } else if (a.mode == B2E_AUTORESET_SAME_STEP) {  // sync_vector_env.py:302-319
       reinterpret_cast<float4*>(a.final_obs)[i] = to_obs(s);
       reset_env_cold(a.state, a.ctrl, a.rng, a.obs, a.n, i, a.low, a.range, a.rng_mode, a.philox_seed,
-                     (uint64_t)(a.env_offset + i), a.call_counter, have_words, w_state, w_inc);
+                     (uint64_t)(a.env_offset + i), a.call_counter);
       return;
     }
   }
@@ -276,13 +241,9 @@ __global__ void __launch_bounds__(1024) cartpole_step_kernel(const CartPoleArgs 
 }
 
 template <typename ActT>
-cudaError_t launch_step(const CartPoleArgs& a, cudaStream_t st, int block) {
-  if (block < 32 || block > 1024 || (block & 31)) block = kStepBlock;
-  // opt-in: measured on B200 at N=65536 (profiles/r2_notes.md) the up-front load wins when the batch is L2-resident (3.03 vs
-  // 3.13 us per launch) but loses on the HBM-cold ring (3.84 vs 3.66 us: +30 % DRAM reads outweigh the saved round trip)
-  static const bool spec = getenv("B2E_CARTPOLE_SPEC_RNG") != nullptr;
-  if (a.n <= kSpecRngMaxEnvs && spec) return launch_pdl(cartpole_step_kernel<ActT, true>, grid_for(a.n, block), block, 0, st, a);
-  return launch_pdl(cartpole_step_kernel<ActT, false>, grid_for(a.n, block), block, 0, st, a);
+cudaError_t launch_step(const CartPoleArgs& a, cudaStream_t st) {
+  cartpole_step_kernel<ActT><<<grid_for(a.n, kStepBlock), kStepBlock, 0, st>>>(a);
+  return cudaGetLastError();
 }
 
 struct RolloutArgs {
@@ -295,7 +256,6 @@ struct RolloutArgs {
 // K fused steps: state in registers, [K][n] trajectory streamed out with coalesced stores.
 template <typename ActT, bool kRandom>
 __global__ void __launch_bounds__(kBlock) cartpole_rollout_kernel(const RolloutArgs r) {
-  pdl_prologue();
   const CartPoleArgs& a = r.a;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
@@ -408,8 +368,8 @@ extern "C" int b2e_cartpole_reset(const b2e_batch* b, const b2e_cartpole_cfg* cf
   a.ctrl = ctrl;
   a.rng = rng;
   a.obs = obs;
-  return cuda_status(launch_pdl(cartpole_reset_kernel, grid_for(b->n), kBlock, 0, (cudaStream_t)stream, a),
-                     "b2e_cartpole_reset");
+  cartpole_reset_kernel<<<grid_for(b->n), kBlock, 0, (cudaStream_t)stream>>>(a);
+  return cuda_status(cudaGetLastError(), "b2e_cartpole_reset");
 }
 
 extern "C" int b2e_cartpole_step(const b2e_batch* b, const b2e_cartpole_cfg* cfg, const void* actions, double* state,
@@ -435,9 +395,9 @@ extern "C" int b2e_cartpole_step(const b2e_batch* b, const b2e_cartpole_cfg* cfg
   cudaStream_t st = (cudaStream_t)stream;
   cudaError_t e;
   switch (b->action_dtype) {
-    case B2E_ACT_I64: e = launch_step<int64_t>(a, st, cfg->step_block); break;
-    case B2E_ACT_I32: e = launch_step<int32_t>(a, st, cfg->step_block); break;
-    case B2E_ACT_U8: e = launch_step<uint8_t>(a, st, cfg->step_block); break;
+    case B2E_ACT_I64: e = launch_step<int64_t>(a, st); break;
+    case B2E_ACT_I32: e = launch_step<int32_t>(a, st); break;
+    case B2E_ACT_U8: e = launch_step<uint8_t>(a, st); break;
     default: set_error("b2e_cartpole_step: action_dtype %d is not a discrete dtype", b->action_dtype); return B2E_EINVAL;
   }
   return cuda_status(e, "b2e_cartpole_step");
@@ -471,16 +431,15 @@ extern "C" int b2e_cartpole_rollout(const b2e_batch* b, const b2e_cartpole_cfg* 
   r.reward32 = reward;
   const unsigned grid = grid_for(b->n);
   cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t e;
   if (!actions) {
-    e = launch_pdl(cartpole_rollout_kernel<uint8_t, true>, grid, kBlock, 0, st, r);
+    cartpole_rollout_kernel<uint8_t, true><<<grid, kBlock, 0, st>>>(r);
   } else {
     switch (b->action_dtype) {
-      case B2E_ACT_I64: e = launch_pdl(cartpole_rollout_kernel<int64_t, false>, grid, kBlock, 0, st, r); break;
-      case B2E_ACT_I32: e = launch_pdl(cartpole_rollout_kernel<int32_t, false>, grid, kBlock, 0, st, r); break;
-      case B2E_ACT_U8: e = launch_pdl(cartpole_rollout_kernel<uint8_t, false>, grid, kBlock, 0, st, r); break;
+      case B2E_ACT_I64: cartpole_rollout_kernel<int64_t, false><<<grid, kBlock, 0, st>>>(r); break;
+      case B2E_ACT_I32: cartpole_rollout_kernel<int32_t, false><<<grid, kBlock, 0, st>>>(r); break;
+      case B2E_ACT_U8: cartpole_rollout_kernel<uint8_t, false><<<grid, kBlock, 0, st>>>(r); break;
       default: set_error("b2e_cartpole_rollout: bad action_dtype %d", b->action_dtype); return B2E_EINVAL;
     }
   }
-  return cuda_status(e, "b2e_cartpole_rollout");
+  return cuda_status(cudaGetLastError(), "b2e_cartpole_rollout");
 }

@@ -11,8 +11,6 @@
 #include <stdint.h>
 #include <stdlib.h>
 
-#include <utility>
-
 #include "../../include/b200env.h"
 
 #if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ < 1000)
@@ -29,46 +27,6 @@ int cuda_status(cudaError_t e, const char* fn);
 
 constexpr int kBlock = 256;  // 8 warps; every kernel here is 1 thread/env (or grid-stride), register-light
 inline unsigned grid_for(int64_t n, int block = kBlock) { return (unsigned)((n + block - 1) / block); }
-
-// Programmatic dependent launch (sm_90+), opt-in with B2E_PDL=1: the kernel is launched with the programmatic-stream-
-// serialization attribute, triggers its dependents at once and waits for its predecessor before its first global
-// access, so the launch latency of step k+1 can overlap the execution of step k (also inside captured CUDA graphs).
-// Without the attribute the two griddepcontrol instructions are no-ops.  Measured on B200 (scripts/floor.py): helps
-// chains of tiny launches (N <= 4096: 2.05 vs 2.21 us) but hurts at N >= 65536 (4.07 vs 3.27 us), hence opt-in.
-__device__ __forceinline__ void pdl_prologue() {
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t stream,
-                              Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(block);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  static const bool pdl = getenv("B2E_PDL") != nullptr;  // opt-in: measured slower at N >= 65536 (DESIGN.md)
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-
-// Sparse lane mapping for the divergent, latency-bound physics kernels: only the first `lanes` lanes of every warp own
-// an env (env = warp * lanes + lane).  Fewer envs per warp = fewer distinct control paths serialised inside a warp and
-// more warps to hide latency when the batch alone cannot fill the machine.
-__device__ __forceinline__ int64_t sparse_env_index(int lanes) {
-  const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = (int)(gtid & 31);
-  return lane < lanes ? (gtid >> 5) * lanes + lane : -1;
-}
-inline unsigned sparse_grid(int64_t n, int lanes, int block) {
-  const int64_t warps = (n + lanes - 1) / lanes;
-  return (unsigned)((warps * 32 + block - 1) / block);
-}
 
 // ---------------------------------------------------------------------------------------------------------------
 // Scheduling helper shared by the physics families: order[] = env indices bucket-sorted by a small integer key

@@ -94,7 +94,6 @@ __device__ __forceinline__ double philox_u(const LakeArgs& a, int64_t i, uint64_
 }
 
 __global__ void __launch_bounds__(kBlock) frozenlake_reset_kernel(const LakeArgs a) {
-  pdl_prologue();
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.n) return;
   if (a.mask != nullptr && a.mask[i] == 0) return;
@@ -115,7 +114,6 @@ __global__ void __launch_bounds__(kBlock) frozenlake_reset_kernel(const LakeArgs
 
 template <typename ActT>
 __global__ void __launch_bounds__(kBlock) frozenlake_step_kernel(const LakeArgs a) {
-  pdl_prologue();
   const uint32_t* t = stage_table(a);
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += (int64_t)gridDim.x * blockDim.x) {
     // all loads first (one DRAM round trip), then the arithmetic
@@ -169,7 +167,6 @@ __global__ void __launch_bounds__(kBlock) frozenlake_step_kernel(const LakeArgs 
 // K fused steps, state + RNG in registers, [K][n] trajectory streamed out
 template <typename ActT, bool kRandom>
 __global__ void __launch_bounds__(kBlock) frozenlake_rollout_kernel(const LakeArgs a) {
-  pdl_prologue();
   const uint32_t* t = stage_table(a);
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += (int64_t)gridDim.x * blockDim.x) {
     int32_t c = a.ctrl[i];
@@ -229,12 +226,11 @@ size_t table_smem_bytes(const LakeArgs& a) {
 
 // Launch geometry: one env per thread (grid = ceil(n / 256)) by default.  A capped grid-stride launch (8 CTAs per SM,
 // table staged once per CTA) was measured slower at N = 1,048,576 because 1M / 303k threads = 3.46 passes leaves the
-// last pass half empty; staging 3 KB per CTA from L2 is cheap.  B2E_LAKE_PERSISTENT=1 restores the capped grid.
+// last pass half empty; staging 3 KB per CTA from L2 is cheap.
 unsigned persistent_grid(int64_t n, size_t table_bytes) {
   // small tables (FrozenLake 8x8: 3 KB): one env per thread; big tables (Taxi: 36 KB) amortise the staging over a
   // grid-stride loop -- measured at N = 8M: Taxi 581 us plain grid (staging 140 B/env of extra L2 traffic)
-  static const bool capped = getenv("B2E_LAKE_PERSISTENT") != nullptr;
-  if (!capped && table_bytes <= 8192) return grid_for(n);
+  if (table_bytes <= 8192) return grid_for(n);
   static int sms = 0;
   if (sms == 0) {
     int dev = 0;
@@ -304,8 +300,8 @@ extern "C" int b2e_frozenlake_reset(const b2e_batch* b, const b2e_frozenlake_cfg
   a.rng = rng;
   a.obs = obs;
   a.prob_out = prob;
-  return cuda_status(launch_pdl(frozenlake_reset_kernel, grid_for(b->n), kBlock, 0, (cudaStream_t)stream, a),
-                     "b2e_frozenlake_reset");
+  frozenlake_reset_kernel<<<grid_for(b->n), kBlock, 0, (cudaStream_t)stream>>>(a);
+  return cuda_status(cudaGetLastError(), "b2e_frozenlake_reset");
 }
 
 extern "C" int b2e_frozenlake_step(const b2e_batch* b, const b2e_frozenlake_cfg* cfg, const void* actions,
@@ -335,12 +331,11 @@ extern "C" int b2e_frozenlake_step(const b2e_batch* b, const b2e_frozenlake_cfg*
   const size_t smem = table_smem_bytes(a);
   const unsigned grid = persistent_grid(b->n, smem);
   cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t ce = cudaSuccess;
   if (int e = launch_by_dtype(b->action_dtype, "b2e_frozenlake_step", [&](auto tag) {
-        ce = launch_pdl(frozenlake_step_kernel<decltype(tag)>, grid, kBlock, smem, st, a);
+        frozenlake_step_kernel<decltype(tag)><<<grid, kBlock, smem, st>>>(a);
       }))
     return e;
-  return cuda_status(ce, "b2e_frozenlake_step");
+  return cuda_status(cudaGetLastError(), "b2e_frozenlake_step");
 }
 
 extern "C" int b2e_frozenlake_rollout(const b2e_batch* b, const b2e_frozenlake_cfg* cfg, int32_t K,
@@ -372,13 +367,12 @@ extern "C" int b2e_frozenlake_rollout(const b2e_batch* b, const b2e_frozenlake_c
   const size_t smem = table_smem_bytes(a);
   const unsigned grid = persistent_grid(b->n, smem);
   cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t ce = cudaSuccess;
   if (!actions) {
-    ce = launch_pdl(frozenlake_rollout_kernel<uint8_t, true>, grid, kBlock, smem, st, a);
+    frozenlake_rollout_kernel<uint8_t, true><<<grid, kBlock, smem, st>>>(a);
   } else if (int e = launch_by_dtype(b->action_dtype, "b2e_frozenlake_rollout", [&](auto tag) {
-               ce = launch_pdl(frozenlake_rollout_kernel<decltype(tag), false>, grid, kBlock, smem, st, a);
+               frozenlake_rollout_kernel<decltype(tag), false><<<grid, kBlock, smem, st>>>(a);
              })) {
     return e;
   }
-  return cuda_status(ce, "b2e_frozenlake_rollout");
+  return cuda_status(cudaGetLastError(), "b2e_frozenlake_rollout");
 }

@@ -973,7 +973,7 @@ int upload_model() {
 // ---- kernels -------------------------------------------------------------------------------------------------------------------
 struct HumanoidArgs {
   int64_t n, env_offset;
-  int32_t max_steps, mode, rng_mode, lanes, frame_skip, terminate_when_unhealthy, cta_sync;
+  int32_t max_steps, mode, rng_mode, frame_skip, terminate_when_unhealthy;
   uint64_t philox_seed, call_counter;
   double noise, w_forward, w_ctrl, w_contact, contact_max, healthy_reward, z_min, z_max;
   double* __restrict__ qpos;   // [24][n]
@@ -1067,14 +1067,12 @@ __device__ void store_state(const HumanoidArgs& a, int64_t i, const HData& d) {
 }
 
 constexpr int kHumanoidBlock = 32;
-constexpr int kWarpEnvsPerCta = 10;  // warp mapping: envs (warps) per CTA unless b2e_humanoid_cfg.envs_per_cta says otherwise
+constexpr int kWarpEnvsPerCta = 10;  // warp mapping: envs (warps) per CTA; N=8192: 8 per CTA 8.4 ms, 10 per CTA 7.5 ms
                                      // (10 x 20.2 KB + the 12.9 KB model = 215 KB of the 227 KB an sm_100a CTA can have)
-constexpr bool kHumanoidDefaultWarp = true;   // warp per env is the default mapping (thread per env: impl = 1)
-constexpr int kHumanoidLanes = 32;  // default envs per warp (b2e_humanoid_cfg.lanes_per_warp overrides)
 
 __global__ void __launch_bounds__(kHumanoidBlock) humanoid_reset_kernel(const HumanoidArgs a) {
-  const int64_t i = sparse_env_index(a.lanes);
-  if (i < 0 || i >= a.n) return;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
   if (a.mask != nullptr && a.mask[i] == 0) return;
   HData d;
   d.overflow = 0;
@@ -1090,8 +1088,8 @@ __global__ void __launch_bounds__(kHumanoidBlock) humanoid_reset_kernel(const Hu
 
 template <typename ActT>
 __global__ void __launch_bounds__(kHumanoidBlock) humanoid_step_kernel(const HumanoidArgs a) {
-  const int64_t i = sparse_env_index(a.lanes);
-  if (i < 0 || i >= a.n) return;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
   const HModel& m = g_hmodel;
   const int32_t c = a.ctrl[i];
   HData d;
@@ -1166,10 +1164,12 @@ __global__ void __launch_bounds__(kHumanoidBlock) humanoid_step_kernel(const Hum
 
 #include "humanoid_warp.cuh"  // warp-per-env mapping of the same physics (shares every HD helper above)
 
-static_assert(sizeof(WModel) + 10 * sizeof(WS) <= 227 * 1024, "10 envs per CTA must fit the 227 KB of shared memory an sm_100a CTA can opt in to");
+static_assert(sizeof(WModel) + kWarpEnvsPerCta * sizeof(WS) <= 227 * 1024,
+              "10 envs per CTA must fit the 227 KB of shared memory an sm_100a CTA can opt in to");
 
-template <typename ActT, int W>
+template <typename ActT>
 int launch_warp_step(const HumanoidArgs& a, cudaStream_t s) {
+  constexpr int W = kWarpEnvsPerCta;
   // opt in to > 48 KB of dynamic shared memory once per instantiation AND device (the attribute is per device/context)
   static std::atomic<bool> configured[64];
   const int smem = (int)sizeof(WModel) + W * (int)sizeof(WS);
@@ -1184,9 +1184,6 @@ int launch_warp_step(const HumanoidArgs& a, cudaStream_t s) {
   humanoid_step_warp_kernel<ActT, W><<<(unsigned)((a.n + W - 1) / W), 32 * W, smem, s>>>(a);
   return cuda_status(cudaGetLastError(), "b2e_humanoid_step");
 }
-
-// implementation choice: b2e_humanoid_cfg.impl 1 = thread per env, 2 = warp per env, 0 = library default
-inline bool use_warp_impl(const b2e_humanoid_cfg* cfg) { return cfg->impl == 2 || (cfg->impl == 0 && kHumanoidDefaultWarp); }
 
 int fill(const b2e_batch* b, const b2e_humanoid_cfg* cfg, const b2e_humanoid_state* st, HumanoidArgs& a, const char* fn) {
   if (int e = check_batch(b, fn)) return e;
@@ -1203,8 +1200,6 @@ int fill(const b2e_batch* b, const b2e_humanoid_cfg* cfg, const b2e_humanoid_sta
   a.n = b->n; a.env_offset = b->env_offset; a.max_steps = b->max_episode_steps; a.mode = b->autoreset_mode;
   a.rng_mode = b->rng_mode; a.philox_seed = b->philox_seed; a.call_counter = b->call_counter;
   a.frame_skip = cfg->frame_skip; a.terminate_when_unhealthy = cfg->terminate_when_unhealthy;
-  a.cta_sync = 0;
-  a.lanes = (cfg->lanes_per_warp >= 1 && cfg->lanes_per_warp <= 32) ? cfg->lanes_per_warp : kHumanoidLanes;
   a.noise = cfg->reset_noise_scale; a.w_forward = cfg->forward_reward_weight; a.w_ctrl = cfg->ctrl_cost_weight;
   a.w_contact = cfg->contact_cost_weight; a.contact_max = cfg->contact_cost_max; a.healthy_reward = cfg->healthy_reward;
   a.z_min = cfg->healthy_z_min; a.z_max = cfg->healthy_z_max;
@@ -1243,10 +1238,10 @@ extern "C" int b2e_humanoid_reset(const b2e_batch* b, const b2e_humanoid_cfg* cf
   }
   if (b->n == 0) return 0;
   a.mask = mask; a.obs = obs; a.info = info;
-  if (use_warp_impl(cfg))
-    humanoid_reset_warp_kernel<<<(unsigned)b->n, 32, 0, (cudaStream_t)stream>>>(a);
+  if (cfg->impl == 1)
+    humanoid_reset_kernel<<<grid_for(b->n, kHumanoidBlock), kHumanoidBlock, 0, (cudaStream_t)stream>>>(a);
   else
-    humanoid_reset_kernel<<<sparse_grid(b->n, a.lanes, kHumanoidBlock), kHumanoidBlock, 0, (cudaStream_t)stream>>>(a);
+    humanoid_reset_warp_kernel<<<(unsigned)b->n, 32, 0, (cudaStream_t)stream>>>(a);
   return cuda_status(cudaGetLastError(), "b2e_humanoid_reset");
 }
 
@@ -1263,29 +1258,15 @@ extern "C" int b2e_humanoid_step(const b2e_batch* b, const b2e_humanoid_cfg* cfg
   if (b->n == 0) return 0;
   a.actions = actions; a.obs = obs; a.reward = reward; a.term = terminated; a.trunc = truncated; a.info = info;
   a.final_obs = final_obs;
-  const unsigned grid = sparse_grid(b->n, a.lanes, kHumanoidBlock);
   cudaStream_t s = (cudaStream_t)stream;
-  if (use_warp_impl(cfg)) {
-    const int W = cfg->envs_per_cta > 0 ? cfg->envs_per_cta : kWarpEnvsPerCta;
-    // schedule bits (tuning knobs, results never change): 1 = no CTA barrier, 2 = no work grouping, 4 = barrier once per
-    // mj_step instead of before every mj_forward, 8 = no barrier but keep the grouping
-    a.cta_sync = (W > 1 && !(cfg->schedule & (1 | 8))) ? ((cfg->schedule & 4) ? 2 : 1) : 0;
-    if ((!a.cta_sync && !(cfg->schedule & 8)) || (cfg->schedule & 2)) a.order = nullptr;  // grouping matters to warps that wait for each other
-    const bool f64 = b->action_dtype == B2E_ACT_F64;
-    if (b->action_dtype != B2E_ACT_F32 && !f64) {
-      set_error("b2e_humanoid_step: action_dtype %d is not a float dtype", b->action_dtype);
-      return B2E_EINVAL;
+  if (cfg->impl != 1) {
+    switch (b->action_dtype) {
+      case B2E_ACT_F32: return launch_warp_step<float>(a, s);
+      case B2E_ACT_F64: return launch_warp_step<double>(a, s);
+      default: set_error("b2e_humanoid_step: action_dtype %d is not a float dtype", b->action_dtype); return B2E_EINVAL;
     }
-    switch (W) {
-      case 1: return f64 ? launch_warp_step<double, 1>(a, s) : launch_warp_step<float, 1>(a, s);
-      case 2: return f64 ? launch_warp_step<double, 2>(a, s) : launch_warp_step<float, 2>(a, s);
-      case 4: return f64 ? launch_warp_step<double, 4>(a, s) : launch_warp_step<float, 4>(a, s);
-      case 8: return f64 ? launch_warp_step<double, 8>(a, s) : launch_warp_step<float, 8>(a, s);
-      case 10: return f64 ? launch_warp_step<double, 10>(a, s) : launch_warp_step<float, 10>(a, s);
-      default: set_error("b2e_humanoid_step: warp mapping supports 1, 2, 4, 8 or 10 envs per CTA, got %d", W); return B2E_EINVAL;
-    }
-    return cuda_status(cudaGetLastError(), "b2e_humanoid_step");
   }
+  const unsigned grid = grid_for(b->n, kHumanoidBlock);
   switch (b->action_dtype) {
     case B2E_ACT_F32: humanoid_step_kernel<float><<<grid, kHumanoidBlock, 0, s>>>(a); break;
     case B2E_ACT_F64: humanoid_step_kernel<double><<<grid, kHumanoidBlock, 0, s>>>(a); break;

@@ -769,11 +769,11 @@ __global__ void __launch_bounds__(32) humanoid_reset_warp_kernel(const HumanoidA
   }
 }
 
-// W envs per CTA, one warp each (the warps never exchange data; sharing a CTA only co-schedules them).  With a.cta_sync the
-// warps also meet at a CTA barrier before every mj_forward evaluation, so they walk the ~165 KB of code together and share
-// instruction-cache lines (barriers between the stages of mj_forward as well were measured: no further gain).  The
-// barrier is ONE instruction inside a loop that every warp of the CTA runs to the end -- warps without an env and warps
-// whose env only resets in this call skip the work, never the barrier.
+// W envs per CTA, one warp each (the warps never exchange data; sharing a CTA only co-schedules them).  The warps also meet
+// at a CTA barrier before every mj_forward evaluation, so they walk the ~165 KB of code together and share instruction-cache
+// lines (barriers between the stages of mj_forward as well were measured: no further gain; a barrier once per mj_step or
+// none at all was slower, DESIGN.md section 4).  The barrier is ONE instruction inside a loop that every warp of the CTA
+// runs to the end -- warps without an env and warps whose env only resets in this call skip the work, never the barrier.
 template <typename ActT, int W>
 __global__ void __launch_bounds__(32 * W) humanoid_step_warp_kernel(const HumanoidArgs a) {
   extern __shared__ __align__(16) unsigned char w_smem[];
@@ -784,7 +784,6 @@ __global__ void __launch_bounds__(32 * W) humanoid_step_warp_kernel(const Humano
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t slot = (int64_t)blockIdx.x * W + warp, n = a.n;
-  const int cta_sync = W > 1 ? a.cta_sync : 0;  // 1: barrier before every mj_forward, 2: once per mj_step
   const bool live = slot < n;
   const int64_t i = !live ? 0 : a.order ? a.order[slot] : slot;  // envs of similar cost share a CTA (they wait for each other)
   WS& w = reinterpret_cast<WS*>(w_smem + sizeof(WModel))[warp];
@@ -810,7 +809,7 @@ __global__ void __launch_bounds__(32 * W) humanoid_step_warp_kernel(const Humano
   for (int k = 0; k < a.frame_skip; ++k) {  // mj_step x frame_skip (mujoco_env.py:150)
 #pragma unroll 1
     for (int st = 0; st < 4; ++st) {
-      if (cta_sync == 1 || (cta_sync == 2 && st == 0)) __syncthreads();
+      __syncthreads();
       if (stepping) w_rk4_stage(wm, w, lane, st);
     }
     if (stepping) w_rk4_finish(wm, w, lane);
@@ -893,7 +892,7 @@ __global__ void __launch_bounds__(32 * W) humanoid_step_warp_kernel(const Humano
   }
 }
 
-// Scheduling helper for the CTA-synchronised step kernel: order[] = env indices bucketed by the solver work of their last
+// Scheduling helper for the step kernel: order[] = env indices bucketed by the solver work of their last
 // step, heaviest first (envs that only reset go last); see group_envs_by_key.
 __global__ void __launch_bounds__(1024) humanoid_group_kernel(const int32_t* __restrict__ work, int32_t* __restrict__ order,
                                                               int64_t n) {

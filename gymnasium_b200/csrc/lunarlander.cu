@@ -1685,7 +1685,7 @@ DI void world_step(Lander& L, float dt, float dt_ratio, float gravity, bool firs
 // ---- kernel arguments / global layout -------------------------------------------------------------------------------------
 struct LanderArgs {
   int64_t n, env_offset;
-  int32_t max_steps, mode, rng_mode, lanes;
+  int32_t max_steps, mode, rng_mode;
   uint64_t philox_seed, call_counter;
   float gravity;
   int32_t continuous, enable_wind;
@@ -1701,9 +1701,6 @@ struct LanderArgs {
   double* __restrict__ prev_shaping; // [n]
   int32_t* __restrict__ ctrl;
   uint64_t* __restrict__ rng;
-  int32_t* __restrict__ work;        // [n] or null: scheduling key of every env after its last step (see lander_key)
-  int32_t* __restrict__ order;       // [slots] or null: env index (or -1) of every thread slot of a grouped launch
-  int64_t slots;
   float* __restrict__ obs;           // [n][8]
   double* __restrict__ reward;
   uint8_t* __restrict__ term;
@@ -2111,55 +2108,13 @@ DI void write_obs(float* __restrict__ obs, int64_t i, const StepOut& o) {
   p[1] = make_float4(o.obs[4], o.obs[5], o.obs[6], o.obs[7]);
 }
 
-// Scheduling key of an env for its NEXT step: which code paths it will walk (no contact candidates / candidates but flying /
-// resting on n manifolds, joints at their limits or not, a reset call).  With b2e_lunarlander_cfg.grouping the step kernel
-// puts envs with equal keys into the same warp.  Scheduling only: which envs share a warp never changes what an env
-// computes.  (Packing equal keys into FULL warps measured slower on B200 at N=16384, 1434 vs 832 us per launch: the slowest
-// warp sets the launch time, and a warp of 32 near-ground envs runs every loop to the worst trip count among 32 of them.)
-DI int lander_key(const Lander& L, bool pending) {
-  if (pending) return 63;
-  int touching = 0;
-  for (int k = 0; k < L.nct; ++k) touching += L.ct[k].touching;
-  const int lim = (L.j[0].limit_state != 0 ? 1 : 0) | (L.j[1].limit_state != 0 ? 2 : 0);
-  const int group = !L.awake ? 0 : L.nct == 0 ? 1 : 2 + min(touching, 12);  // asleep | free flight | near / on the ground
-  return group * 4 + lim;  // <= 59
-}
-// Layout of the step kernel's thread slots when grouping is on: envs in free flight (and asleep / resetting ones) are packed
-// 32 per warp; every env near or on the ground (contact candidates exist: collide, TOI, contact rows) gets a SPARSE warp
-// shared with at most `hl - 1` others, the remaining lanes stay idle.  A launch lasts as long as its slowest warp, and a
-// warp walks the union of its lanes' paths with the longest trip count of every loop, so the expensive envs should wait
-// for as few neighbours as possible, while the cheap, uniform ones fill whole warps.  order[slot] = env index or -1.
-DI bool lander_key_heavy(int key) { return key != 63 && key >= 8; }
-__global__ void __launch_bounds__(1024) lunarlander_group_kernel(const int32_t* __restrict__ work, int32_t* __restrict__ order,
-                                                                 int64_t n, int64_t slots, int hl) {
-  __shared__ int n_light, c_light, c_heavy;
-  const int tid = threadIdx.x, nt = blockDim.x;
-  if (tid == 0) n_light = c_light = c_heavy = 0;
-  for (int64_t s = tid; s < slots; s += nt) order[s] = -1;
-  __syncthreads();
-  int mine = 0;
-  for (int64_t i = tid; i < n; i += nt) mine += lander_key_heavy(work[i]) ? 0 : 1;
-  if (mine) atomicAdd(&n_light, mine);
-  __syncthreads();
-  const int64_t heavy_base = ((int64_t)(n_light + 31) / 32) * 32;
-  for (int64_t i = tid; i < n; i += nt) {
-    if (lander_key_heavy(work[i])) {
-      const int j = atomicAdd(&c_heavy, 1);
-      order[heavy_base + (int64_t)(j / hl) * 32 + (j % hl)] = (int32_t)i;
-    } else {
-      order[atomicAdd(&c_light, 1)] = (int32_t)i;
-    }
-  }
-}
-inline int lander_group_lanes(int g) { return g < 4 ? 4 : (g > 32 ? 32 : g); }  // order[] holds 9 n + 64 slots: >= 4 lanes per sparse warp
-inline int64_t lander_group_slots(int64_t n, int hl) { return 32 * ((n + 31) / 32 + (n + hl - 1) / hl); }
-
+// One thread per env.  Grouping envs by the code paths they will walk (into full or sparse warps) was measured slower or
+// no faster on B200 at N=16384 (DESIGN.md section 4, profiles/r2_notes.md).
 constexpr int kLanderBlock = 64;  // small CTAs: every SM gets work; the kernel is latency- not occupancy-bound
-constexpr int kLanderLanes = 32;  // default envs per warp (b2e_lunarlander_cfg.lanes_per_warp overrides)
 
 __global__ void __launch_bounds__(kLanderBlock) lunarlander_reset_kernel(const LanderArgs a) {
-  const int64_t i = sparse_env_index(a.lanes);
-  if (i < 0 || i >= a.n) return;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
   if (a.mask != nullptr && a.mask[i] == 0) return;
   Lander L;
   L.overflow = 0;
@@ -2172,22 +2127,13 @@ __global__ void __launch_bounds__(kLanderBlock) lunarlander_reset_kernel(const L
   store_draws(a, i, D);
   store_state(a, i, L);
   a.ctrl[i] = 0;
-  if (a.work) a.work[i] = lander_key(L, false);
   write_obs(a.obs, i, o);
 }
 
 template <typename ActT>
 __global__ void __launch_bounds__(kLanderBlock) lunarlander_step_kernel(const LanderArgs a) {
-  int64_t i;
-  if (a.order) {  // grouped launch: dense warps of cheap envs, sparse warps for the expensive ones (lunarlander_group_kernel)
-    const int64_t slot = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot >= a.slots) return;
-    i = a.order[slot];
-    if (i < 0) return;
-  } else {
-    i = sparse_env_index(a.lanes);
-    if (i < 0 || i >= a.n) return;
-  }
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
   const int32_t c = a.ctrl[i];
   int action;
   double a0, a1;
@@ -2236,7 +2182,6 @@ __global__ void __launch_bounds__(kLanderBlock) lunarlander_step_kernel(const La
   store_draws(a, i, D);
   store_state(a, i, L);
   a.ctrl[i] = cn;
-  if (a.work) a.work[i] = lander_key(L, ctrl_pending(cn));
   write_obs(a.obs, i, o);
 }
 
@@ -2407,7 +2352,6 @@ int fill(const b2e_batch* b, const b2e_lunarlander_cfg* cfg, const b2e_lunarland
   a.philox_seed = b->philox_seed;
   a.call_counter = b->call_counter;
   a.gravity = (float)cfg->gravity;
-  a.lanes = (cfg->lanes_per_warp >= 1 && cfg->lanes_per_warp <= 32) ? cfg->lanes_per_warp : kLanderLanes;
   a.bodies = st->bodies;
   a.joints = st->joints;
   a.terrain = st->terrain;
@@ -2417,9 +2361,6 @@ int fill(const b2e_batch* b, const b2e_lunarlander_cfg* cfg, const b2e_lunarland
   a.prev_shaping = st->prev_shaping;
   a.ctrl = st->ctrl;
   a.rng = st->rng;
-  a.work = st->work;
-  a.order = (st->work && st->order && cfg->grouping > 0) ? st->order : nullptr;
-  a.slots = a.order ? lander_group_slots(b->n, lander_group_lanes(cfg->grouping)) : 0;
   return upload_model();
 }
 
@@ -2441,7 +2382,7 @@ extern "C" int b2e_lunarlander_reset(const b2e_batch* b, const b2e_lunarlander_c
   if (b->n == 0) return 0;
   a.mask = mask;
   a.obs = obs;
-  lunarlander_reset_kernel<<<sparse_grid(b->n, a.lanes, kLanderBlock), kLanderBlock, 0, (cudaStream_t)stream>>>(a);
+  lunarlander_reset_kernel<<<grid_for(b->n, kLanderBlock), kLanderBlock, 0, (cudaStream_t)stream>>>(a);
   return cuda_status(cudaGetLastError(), "b2e_lunarlander_reset");
 }
 
@@ -2462,9 +2403,8 @@ extern "C" int b2e_lunarlander_step(const b2e_batch* b, const b2e_lunarlander_cf
   a.term = terminated;
   a.trunc = truncated;
   a.final_obs = final_obs;
-  const unsigned grid = a.order ? (unsigned)((a.slots + kLanderBlock - 1) / kLanderBlock) : sparse_grid(b->n, a.lanes, kLanderBlock);
+  const unsigned grid = grid_for(b->n, kLanderBlock);
   cudaStream_t s = (cudaStream_t)stream;
-  if (a.order) lunarlander_group_kernel<<<1, 1024, 0, s>>>(a.work, a.order, a.n, a.slots, lander_group_lanes(cfg->grouping));
   if (cfg->continuous) {  // actions [n][2] float32 / float64 in [-1, 1] (clipped in-kernel like the reference, :510)
     switch (b->action_dtype) {
       case B2E_ACT_F32: lunarlander_step_kernel<float><<<grid, kLanderBlock, 0, s>>>(a); break;

@@ -1074,7 +1074,7 @@ constexpr int kObs = NQ - 1 + NV;
 constexpr int kInfo = 6;  // info rows: x_position, z_distance_from_origin, x_velocity, reward_forward, reward_ctrl, reward_survive
 struct HopperArgs {
   int64_t n, env_offset;
-  int32_t max_steps, mode, rng_mode, lanes, frame_skip, terminate_when_unhealthy;
+  int32_t max_steps, mode, rng_mode, frame_skip, terminate_when_unhealthy;
   uint64_t philox_seed, call_counter;
   double noise, w_forward, w_ctrl, healthy_reward, z_min, z_max, angle_min, angle_max, state_min, state_max;
   double* __restrict__ qpos;  // [6][n]
@@ -1252,7 +1252,6 @@ __device__ void store_state(const HopperArgs& a, int64_t i, const HData& d) {
 }
 
 constexpr int kHopperBlock = 64;
-constexpr int kHopperLanes = 32;  // default envs per warp (b2e_mjplanar_cfg.lanes_per_warp overrides)
 
 __device__ PDraws make_draws(const HopperArgs& a, int64_t i) {
   PDraws D;
@@ -1262,8 +1261,8 @@ __device__ PDraws make_draws(const HopperArgs& a, int64_t i) {
 }
 
 __global__ void __launch_bounds__(kHopperBlock) hopper_reset_kernel(const HopperArgs a) {
-  const int64_t i = sparse_env_index(a.lanes);
-  if (i < 0 || i >= a.n) return;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
   if (a.mask != nullptr && a.mask[i] == 0) return;
   HData d;
   d.overflow = 0;
@@ -1277,8 +1276,8 @@ __global__ void __launch_bounds__(kHopperBlock) hopper_reset_kernel(const Hopper
 
 template <typename ActT>
 __global__ void __launch_bounds__(kHopperBlock) hopper_step_kernel(const HopperArgs a) {
-  const int64_t i = sparse_env_index(a.lanes);
-  if (i < 0 || i >= a.n) return;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= a.n) return;
   const HModel& m = g_pmodel;
   const int32_t c = a.ctrl[i];
   HData d;
@@ -1387,7 +1386,6 @@ int fill(const b2e_batch* b, const b2e_mjplanar_cfg* cfg, const b2e_mjplanar_sta
   a.n = b->n; a.env_offset = b->env_offset; a.max_steps = b->max_episode_steps; a.mode = b->autoreset_mode;
   a.rng_mode = b->rng_mode; a.philox_seed = b->philox_seed; a.call_counter = b->call_counter;
   a.frame_skip = cfg->frame_skip; a.terminate_when_unhealthy = cfg->terminate_when_unhealthy;
-  a.lanes = (cfg->lanes_per_warp >= 1 && cfg->lanes_per_warp <= 32) ? cfg->lanes_per_warp : kHopperLanes;
   a.noise = cfg->reset_noise_scale; a.w_forward = cfg->forward_reward_weight; a.w_ctrl = cfg->ctrl_cost_weight;
   a.healthy_reward = cfg->healthy_reward;
   a.z_min = cfg->healthy_z_min; a.z_max = cfg->healthy_z_max;
@@ -1427,7 +1425,7 @@ extern "C" int MJC_API(reset)(const b2e_batch* b, const b2e_mjplanar_cfg* cfg, c
   }
   if (b->n == 0) return 0;
   a.mask = mask; a.obs = obs; a.info = info;
-  hopper_reset_kernel<<<sparse_grid(b->n, a.lanes, kHopperBlock), kHopperBlock, 0, (cudaStream_t)stream>>>(a);
+  hopper_reset_kernel<<<grid_for(b->n, kHopperBlock), kHopperBlock, 0, (cudaStream_t)stream>>>(a);
   return cuda_status(cudaGetLastError(), "b2e_" MJC_NAME "_reset");
 }
 
@@ -1444,7 +1442,7 @@ extern "C" int MJC_API(step)(const b2e_batch* b, const b2e_mjplanar_cfg* cfg, co
   if (b->n == 0) return 0;
   a.actions = actions; a.obs = obs; a.reward = reward; a.term = terminated; a.trunc = truncated; a.info = info;
   a.final_obs = final_obs;
-  const unsigned grid = sparse_grid(b->n, a.lanes, kHopperBlock);
+  const unsigned grid = grid_for(b->n, kHopperBlock);
   cudaStream_t s = (cudaStream_t)stream;
   switch (b->action_dtype) {
     case B2E_ACT_F32: hopper_step_kernel<float><<<grid, kHopperBlock, 0, s>>>(a); break;

@@ -143,8 +143,9 @@ class HostBatch:
             self.keys.append((key, gshape, npdt, off, rowb, rows))
             off = (off + int(np.prod(gshape, dtype=np.int64)) * npdt.itemsize + 255) // 256 * 256
         self.slot_bytes = max(off, 256)
-        # counters (one line per rank + the ack line), then per rank a line-aligned ring of sequence-word SOURCES: the value
-        # step k publishes is written there by the host and copied behind the data by the same stream (pinned -> pinned)
+        # counters (one line per rank + the ack line), then per rank a line-aligned ring of sequence-word SOURCES for the
+        # copy-engine landing (HostBatchPipeline's Python path): the value step k publishes is written there by the host and
+        # copied behind the data by the same stream
         self.src_ring = 2 * self.depth + 2
         self._src_off = self.LINE * (self.world + 1)
         self._src_stride = (8 * self.src_ring + self.LINE - 1) // self.LINE * self.LINE
@@ -241,11 +242,6 @@ class HostBatch:
     def seq_addr(self, rank: int | None = None) -> int:
         r = self.rank if rank is None else rank
         return self._addr + r * self.LINE
-
-    def seq_slot_source(self, j: int) -> int:
-        """Address of the page-locked word slot j's sequence copy reads (fast path: written by ``b2e_pipe_submit`` itself once
-        the slot has been released, so one fixed word per slot is enough)."""
-        return self._addr + self._src_off + self._src_stride * self.rank + 8 * (j % self.src_ring)
 
     def seq_source(self, k: int) -> int:
         """Writes k+1 into this rank's source ring and returns its address (the last copy segment of step k reads it)."""
@@ -345,8 +341,9 @@ class _CallRecorder:
 
 class HostBatchPipeline:
     """Pipelined end-to-end stepping of one shard.  ``submit(host_actions)`` enqueues the pinned H2D copy of the actions and
-    the fused step launch on the caller's stream and, on a copy stream, the D2H copies of the step outputs into this rank's
-    rows of the shared :class:`HostBatch` followed by its 8-byte sequence word -- no host synchronisation.  ``consume(k)``
+    the fused step launch on the caller's stream and, on a copy stream, the landing of the step outputs into this rank's
+    rows of the shared :class:`HostBatch` followed by its 8-byte sequence word -- no host synchronisation.  The fast path
+    (numpy-parity RNG) lands them with one kernel; the Python path (``fast=False``) with the copy engine.  ``consume(k)``
     (consumer rank) waits until every rank's rows of step k have landed and returns numpy views of the whole batch.  The
     copies of step k overlap the kernel of step k+1 (the env rotates over `depth` output buffers).
 
@@ -355,7 +352,7 @@ class HostBatchPipeline:
     """
 
     def __init__(self, env, world_size: int, rank: int, total_envs: int | None = None, tag: str = "0", depth: int = 3,
-                 mode: str = "dma", consumer: int = 0, fast: bool = True, landing: str | None = None):
+                 mode: str = "dma", consumer: int = 0, fast: bool = True):
         if env.output != "torch" or env.copy or env.out_buffers < depth:
             raise ValueError("HostBatchPipeline needs an env made with output='torch', copy=False, out_buffers >= depth")
         if mode not in ("dma", "nccl"):
@@ -397,11 +394,9 @@ class HostBatchPipeline:
         # recorded step call(s) -- set up lazily at the first submit, when the action dtype / shape is known
         self._fast = None if (mode == "dma" and fast and env.rng_mode == "numpy") else False
         self._slots = None
-        # how a step's rows reach the host batch on the fast path: "kernel" (one launch, SM stores over PCIe, publishes the
-        # sequence word itself), "graph" (the copy engine's per-key copies as one CUDA graph), "copies" (one call per key)
-        self.landing = os.environ.get("B2E_PIPE_LANDING", "kernel") if landing is None else landing
-        if self.landing not in ("kernel", "graph", "copies"):
-            raise ValueError(f"landing must be 'kernel', 'graph' or 'copies', got {self.landing!r}")
+        # the fast path lands a step's rows with one kernel launch (SM stores over PCIe, then the sequence word); the copy
+        # engine's per-key copies, alone or as one CUDA graph, were slower (DESIGN.md section 6)
+        self.landing = "kernel"
         self._pinned_ptrs: set = set()
         self._pinned_keep: list = []
 
@@ -490,20 +485,18 @@ class HostBatchPipeline:
                 for i, wd in enumerate(words):
                     c.args[i] = wd
             seg_list = self.host.segments(j, self.rank, {e[0]: out[e[0]].data_ptr() for e in self.layout})
+            # the two publication segments of the copy-engine path: the landing kernel stores the sequence word itself and
+            # takes only its address from the last one
             bounce = self._seq_dev[j:].data_ptr()
-            seg_list.append((bounce, 0, 0, 0, 8, 1))  # source patched per step by b2e_pipe_submit
+            seg_list.append((bounce, 0, 0, 0, 8, 1))
             seg_list.append((self.host.seq_addr(), bounce, 0, 0, 8, 1))
             segs = (L.CopySeg * len(seg_list))(*[L.CopySeg(*sg) for sg in seg_list])
             sl = slots[j]
             sl.staging_host, sl.actions_dev, sl.action_bytes = staging.data_ptr(), act_dev.data_ptr(), a.nbytes
             sl.calls, sl.ncalls = calls, len(rec.calls)
             sl.segs, sl.nsegs = segs, len(seg_list)
-            sl.seq_src = self.host.seq_slot_source(j)
             L.check(self._lib.b2e_pipe_slot_init(C.byref(sl)), "b2e_pipe_slot_init")
-            if self.landing == "kernel":
-                L.check(self._lib.b2e_pipe_slot_land_kernel(C.byref(sl)), "b2e_pipe_slot_land_kernel")
-            elif self.landing == "graph":  # the D2H side of a step becomes ONE cudaGraphLaunch
-                L.check(self._lib.b2e_pipe_slot_capture(C.byref(sl), self._cs_handle), "b2e_pipe_slot_capture")
+            L.check(self._lib.b2e_pipe_slot_land_kernel(C.byref(sl)), "b2e_pipe_slot_land_kernel")
             self._keep += [staging, act_dev, calls, segs]
         self._slots = slots
         self._ack_addr = self.host._addr + self.host.world * self.host.LINE
@@ -527,7 +520,7 @@ class HostBatchPipeline:
             k, j = self.k, self.k % self.depth
             ptr = a.ctypes.data
             st = self._lib.b2e_pipe_submit(self._C.byref(self._slots[j]), ptr, self._main_handle, self._cs_handle,
-                                           self._ack_addr, k - self.depth + 1, self._slots[j].seq_src, k + 1,
+                                           self._ack_addr, k - self.depth + 1, k + 1,
                                            1 if ptr in self._pinned_ptrs else 0, 120.0)
             if st:
                 self._lib_mod.check(st, "b2e_pipe_submit")

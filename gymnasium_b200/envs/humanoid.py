@@ -8,7 +8,6 @@ Numeric parity with the real MuJoCo wheel is unpinned (it cannot be installed he
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import numpy as np
 import torch
@@ -19,7 +18,7 @@ from ..vector_env import B200VectorEnv, ptr
 
 INFO_KEYS = ("x_position", "y_position", "tendon_length", "tendon_velocity", "distance_from_origin", "x_velocity",
              "y_velocity", "reward_survive", "reward_forward", "reward_ctrl", "reward_contact")
-_IMPLS = {"default": 0, "thread": 1, "warp": 2}  # b2e_humanoid_cfg.impl: kernel mapping (same results bit for bit)
+_IMPLS = {"warp": 0, "thread": 1}  # b2e_humanoid_cfg.impl: kernel mapping (same results bit for bit)
 OBS_SIZE = 22 + 23 + 130 + 78 + 17 + 78  # humanoid_v5.py:376-393
 
 
@@ -38,8 +37,7 @@ class HumanoidVectorEnv(B200VectorEnv):
                  exclude_current_positions_from_observation: bool = True, include_cinert_in_observation: bool = True,
                  include_cvel_in_observation: bool = True, include_qfrc_actuator_in_observation: bool = True,
                  include_cfrc_ext_in_observation: bool = True, render_mode: str | None = None,
-                 impl: str | None = None, **engine_kwargs):
-        impl = impl or os.environ.get("B2E_HUMANOID_IMPL") or "default"
+                 impl: str = "warp", **engine_kwargs):
         if impl not in _IMPLS:
             raise ValueError(f"impl must be one of {sorted(_IMPLS)}, got {impl!r}")
         if xml_file != "humanoid.xml":

@@ -58,8 +58,6 @@ class LunarLanderVectorEnv(B200VectorEnv):
             "contacts": torch.zeros((words, n), dtype=torch.int32, device=dev),
             "flags": torch.zeros(n, dtype=torch.int32, device=dev),
             "prev_shaping": torch.zeros(n, dtype=torch.float64, device=dev),
-            "work": torch.zeros(n, dtype=torch.int32, device=dev),    # scheduling key of every env after its last step
-            "order": torch.zeros(9 * n + 64, dtype=torch.int32, device=dev),  # scratch: thread slot -> env of a grouped launch
         }
         if self.enable_wind:  # wind pattern offsets + the 32-bit word np_random.integers leaves in PCG64's buffer
             self._s["wind"] = torch.zeros((2, n), dtype=torch.int32, device=dev)

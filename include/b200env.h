@@ -93,11 +93,12 @@ int b2e_copy_to_host_async(const b2e_copy_seg* segs, int32_t count, void* stream
  *   staging_host / actions_dev / action_bytes : page-locked staging buffer and the device buffer the step reads actions from
  *   calls / ncalls : the family's step for this output set, recorded as C-ABI calls of THIS header (function address + its
  *                    arguments; every argument of every step entry point is a pointer or an integer, i.e. one machine word)
- *   segs / nsegs   : the landing copies (b2e_copy_seg) of this output set; the last two publish the sequence word
+ *   segs / nsegs   : the output segments (b2e_copy_seg) of this output set, then two 8-byte segments whose last one's
+ *                    host_dst is the rank's sequence word (the landing kernel lands the first nsegs - 2 and stores the word)
  *   ev_*           : cudaEvent_t, owned by the slot (b2e_pipe_slot_init / _destroy)
  * b2e_pipe_submit(slot, host_actions, ...): memcpy into the staging buffer (skipped with B2E_PIPE_ACTIONS_PINNED: the DMA
  * reads the caller's page-locked buffer), async H2D on main_stream, the recorded step,
- * then on copy_stream (ordered after the step) the landing copies -- after the consumer's acknowledgement word *ack_word has
+ * then on copy_stream (ordered after the step) the landing kernel -- after the consumer's acknowledgement word *ack_word has
  * reached need_ack (spin, timeout_s).  Never synchronises a stream; returns B2E_ETIMEOUT if the consumer stalls. */
 typedef struct b2e_call {
   void* fn;
@@ -114,15 +115,10 @@ typedef struct b2e_pipe_slot {
   int32_t ncalls, nsegs;
   void *ev_h2d, *ev_step, *ev_copy;
   int32_t h2d_pending, copy_pending;
-  int64_t* seq_src; /* page-locked word of this slot that the landing graph's sequence copy reads (b2e_pipe_slot_capture) */
-  void* copy_graph; /* cudaGraphExec_t of the landing copies, owned by the slot; NULL = the copies are enqueued one by one */
-  void* land;       /* landing-kernel plan, owned by the slot (b2e_pipe_slot_land_kernel); takes precedence over copy_graph */
+  void* land; /* landing-kernel plan, owned by the slot (b2e_pipe_slot_land_kernel); b2e_pipe_submit needs it */
 } b2e_pipe_slot;
 #define B2E_PIPE_ACTIONS_PINNED 1 /* host_actions is page-locked and stays untouched until the step has landed: no staging copy */
 int b2e_pipe_slot_init(b2e_pipe_slot* slot);
-/* Bakes the slot's landing copies (segs, the sequence word read from slot->seq_src) into one CUDA graph: a step's D2H side is
- * then ONE cudaGraphLaunch instead of nsegs cudaMemcpyAsync calls. */
-int b2e_pipe_slot_capture(b2e_pipe_slot* slot, void* copy_stream);
 /* The landing KERNEL: the slot's output rows are stored into the page-locked host batch by the SMs (zero-copy stores over
  * PCIe, 16 bytes per thread) in ONE launch that also publishes the sequence word (system-scope fence, last CTA stores it) --
  * no per-key copy-engine set-up, no bounce word.  Needs the host batch mapped (b2e_host_register does) and <= 8 output keys. */
@@ -133,11 +129,9 @@ int b2e_land_plan_create(const b2e_copy_seg* segs, int32_t count, int64_t* seq_h
 int b2e_land_plan_launch(void* plan, int64_t seq_value, void* stream);
 int b2e_land_plan_destroy(void* plan);
 int b2e_pipe_slot_destroy(b2e_pipe_slot* slot);
-/* seq_value (= step index + 1) is stored to the sequence word's source -- slot->seq_src with a landing graph, else seq_src --
- * after the wait on *ack_word, i.e. when the copy that published the slot's previous step has read it. */
+/* seq_value (= step index + 1) is the sequence word the landing kernel publishes behind the step's rows. */
 int b2e_pipe_submit(b2e_pipe_slot* slot, const void* host_actions, void* main_stream, void* copy_stream,
-                    const int64_t* ack_word, int64_t need_ack, void* seq_src, int64_t seq_value, int32_t flags,
-                    double timeout_s);
+                    const int64_t* ack_word, int64_t need_ack, int64_t seq_value, int32_t flags, double timeout_s);
 
 /* ---- RNG: gymnasium/utils/seeding.py:39-41 -> numpy SeedSequence -> PCG64 ---------------------------------------
  * rng   : uint64 [2][n][2]  = {state(lo,hi)}[n] then {inc(lo,hi)}[n]
@@ -157,7 +151,6 @@ int b2e_rng_random(const b2e_batch* b, uint64_t* rng, int32_t k, double* out, vo
 typedef struct b2e_cartpole_cfg {
   double reset_low, reset_high; /* cartpole.py:236-241 (+ options low/high, classic_control/utils.py:17-46) */
   int32_t sutton_barto_reward;  /* cartpole.py:205-220 */
-  int32_t step_block;           /* threads per CTA of the step kernel; 0 = library default (tuning knob) */
 } b2e_cartpole_cfg;
 
 /* CartPoleEnv.reset for lanes with mask!=0 (NULL = all); clears elapsed/autoreset; writes obs for those lanes. */
@@ -285,9 +278,6 @@ typedef struct b2e_lunarlander_cfg {
   double gravity;        /* LunarLander(gravity=-10.0) */
   int32_t enable_wind;   /* lunar_lander.py:476-506: wind force / turbulence torque while no leg touches the ground */
   int32_t continuous;    /* lunar_lander.py:509-616: actions float [n][2] = (main throttle, lateral throttle) in [-1, 1] */
-  int32_t lanes_per_warp; /* envs mapped to each warp (1..32); 0 = library default. Fewer lanes = less divergence */
-  int32_t grouping;       /* h > 0: envs in free flight share dense warps, envs near the ground get sparse warps of h lanes (clamped to 4..32)
-                             (needs work/order; scheduling only); 0 = off */
   double wind_power;       /* 15.0 */
   double turbulence_power; /* 1.5 */
 } b2e_lunarlander_cfg;
@@ -302,9 +292,6 @@ typedef struct b2e_lunarlander_state {
   double* prev_shaping;
   int32_t* ctrl;
   uint64_t* rng;
-  int32_t* work;   /* [n] optional (may be NULL with order): scheduling key of every env after its last step */
-  int32_t* order;  /* [9 * n + 64] optional scratch: env index (or -1) of every thread slot of a grouped launch
-                      (scheduling only: results do not depend on it) */
   int32_t* wind;   /* [2][n] wind_idx, torque_idx: offsets into the wind pattern, drawn at reset (enable_wind; else NULL) */
   int64_t* u32buf; /* [n] PCG64's one-word 32-bit buffer (bit 32 = valid) that np_random.integers leaves behind
                       (enable_wind with the numpy RNG; else NULL).  Zero it whenever the streams are re-seeded. */
@@ -339,11 +326,8 @@ typedef struct b2e_humanoid_cfg {
   double healthy_z_min, healthy_z_max; /* (1.0, 2.0) */
   int32_t terminate_when_unhealthy;    /* 1 */
   int32_t frame_skip;                  /* 5 */
-  int32_t lanes_per_warp;              /* thread-per-env mapping: envs per warp (1..32); 0 = library default */
-  int32_t impl;                        /* 0 = library default, 1 = thread per env, 2 = warp per env (shared memory) */
-  int32_t envs_per_cta;                /* warp mapping: 1, 2, 4, 8 or 10 envs (warps) per CTA; 0 = library default */
-  int32_t schedule;                    /* warp mapping, bit 0: no CTA barrier before each mj_forward evaluation,
-                                          bit 1: do not group envs by solver work (both only affect speed) */
+  int32_t impl;                        /* 0 = warp per env (shared memory), 1 = thread per env; results are bit-identical */
+  int32_t _pad;
 } b2e_humanoid_cfg;
 
 typedef struct b2e_humanoid_state {
@@ -387,8 +371,6 @@ typedef struct b2e_mjplanar_cfg {
   double healthy_state_min, healthy_state_max; /* Hopper only: (-100, 100) */
   int32_t terminate_when_unhealthy;            /* 1 */
   int32_t frame_skip;                          /* 4 */
-  int32_t lanes_per_warp;                      /* envs per warp (1..32); 0 = library default */
-  int32_t _pad;
 } b2e_mjplanar_cfg;
 
 typedef struct b2e_mjplanar_state {
@@ -417,7 +399,7 @@ int b2e_walker2d_step(const b2e_batch* b, const b2e_mjplanar_cfg* cfg, const b2e
 /* HalfCheetah-v5: gymnasium/envs/mujoco/half_cheetah_v5.py:220-281, assets/half_cheetah.xml on the same kernels (Euler
  * integrator with implicit joint damping, joint springs, settotalmass 14, per-actuator gears).  nq = nv = 9, nu = 6; cfg uses
  * reset_noise_scale (0.1: uniform on qpos, 0.1 * standard_normal on qvel -- numpy's ziggurat over the env's PCG64 stream),
- * forward_reward_weight (1.0), ctrl_cost_weight (0.1), frame_skip (5), lanes_per_warp.  obs float64 [n][17] = qpos[1:] | qvel;
+ * forward_reward_weight (1.0), ctrl_cost_weight (0.1) and frame_skip (5).  obs float64 [n][17] = qpos[1:] | qvel;
  * never terminates; info rows 0 x_position, 2 x_velocity, 3 reward_forward, 4 reward_ctrl; nbody = 8. */
 int b2e_half_cheetah_model_info(double* body_mass, double* misc, double* invweight);
 int b2e_half_cheetah_reset(const b2e_batch* b, const b2e_mjplanar_cfg* cfg, const b2e_mjplanar_state* st, const uint8_t* mask,
@@ -427,7 +409,7 @@ int b2e_half_cheetah_step(const b2e_batch* b, const b2e_mjplanar_cfg* cfg, const
                           void* stream);
 /* InvertedPendulum-v5: gymnasium/envs/mujoco/inverted_pendulum_v5.py:147-186, assets/inverted_pendulum.xml on the same
  * kernels.  nq = nv = 2 (slider, hinge), nu = 1 (ctrlrange +-3, gear 100), timestep 0.02; cfg uses reset_noise_scale (0.01),
- * frame_skip (2) and lanes_per_warp only.  obs float64 [n][4] = qpos | qvel; reward 1.0 while |angle| <= 0.2 and the state is
+ * and frame_skip (2) only.  obs float64 [n][4] = qpos | qvel; reward 1.0 while |angle| <= 0.2 and the state is
  * finite, else 0.0 and terminated; info row 5 = reward_survive (rows 0-4 zero); nbody = 3. */
 int b2e_inverted_pendulum_model_info(double* body_mass, double* misc, double* invweight);
 int b2e_inverted_pendulum_reset(const b2e_batch* b, const b2e_mjplanar_cfg* cfg, const b2e_mjplanar_state* st,

@@ -20,7 +20,6 @@ def chain(env, acts, L=64, reps=50):
     b.record(); torch.cuda.synchronize()
     return a.elapsed_time(b) * 1e3 / (reps * L)
 
-print("PDL disabled" if os.environ.get("B2E_NO_PDL") else "PDL enabled")
 for fam, kw, na in [("CartPole-v1", {}, 2), ("FrozenLake-v1", {"map_name": "8x8"}, 4)]:
     for n in [32, 4096, 65536, 262144]:
         env = gymnasium_b200.make_vec(fam, num_envs=n, copy=False, **kw)

@@ -107,40 +107,38 @@ def main():
                       f"{nb / 1e6:.2f} MB copy, {per:5.1f} GB/s per rank, {per * world:6.1f} GB/s aggregate", flush=True)
         if arr is not None:
             lib.b2e_host_unregister(arr.ctypes.data)
-    # the landing kernel (SM stores into the mapped shared file + sequence word), per grid size
+    # the landing kernel (SM stores into the mapped shared file + sequence word)
     import ctypes as C
 
     mm, arr, ptr = shared("c", False)
     seq_mm = mmap.mmap(-1, 4096)
     seq_np = np.frombuffer(seq_mm, dtype=np.int64)
     _lib.check(lib.b2e_host_register(seq_np.ctypes.data, 4096), "b2e_host_register")
-    for grid in (8, 16, 24, 37, 74, 148, 296):
-        os.environ["B2E_LAND_GRID"] = str(grid)
-        seg = (_lib.CopySeg * 1)()
-        seg[0].host_dst, seg[0].dev_src, seg[0].dst_pitch, seg[0].src_pitch, seg[0].width, seg[0].height = ptr, src.data_ptr(), 0, 0, nb, 1
-        plan = C.c_void_p()
-        _lib.check(lib.b2e_land_plan_create(seg, 1, seq_np.ctypes.data, C.byref(plan)), "b2e_land_plan_create")
-        best = None
-        for rep in range(3):
-            torch.cuda.synchronize()
-            barrier()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            with torch.cuda.stream(s_out):
-                e0.record()
-                for i in range(args.iters):
-                    lib.b2e_land_plan_launch(plan, i + 1, C.c_void_p(s_out.cuda_stream))
-                e1.record()
-            torch.cuda.synchronize()
-            t = torch.tensor([e0.elapsed_time(e1) * 1e-3], dtype=torch.float64, device=dev)
-            if world > 1:
-                dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            best = float(t.item()) if best is None else min(best, float(t.item()))
-        ok = int(seq_np[0]) == args.iters and bool((arr[rank * nb:(rank + 1) * nb] == src.cpu().numpy()).all())
-        if rank == 0:
-            per = nb * args.iters / best / 1e9
-            print(f"world={world} landing kernel, {grid:4d} CTAs x 256        : {best / args.iters * 1e6:7.1f} us per {nb / 1e6:.2f} MB, "
-                  f"{per:5.1f} GB/s per rank, {per * world:6.1f} GB/s aggregate, data+seq {'ok' if ok else 'WRONG'}", flush=True)
-        lib.b2e_land_plan_destroy(plan)
+    seg = (_lib.CopySeg * 1)()
+    seg[0].host_dst, seg[0].dev_src, seg[0].dst_pitch, seg[0].src_pitch, seg[0].width, seg[0].height = ptr, src.data_ptr(), 0, 0, nb, 1
+    plan = C.c_void_p()
+    _lib.check(lib.b2e_land_plan_create(seg, 1, seq_np.ctypes.data, C.byref(plan)), "b2e_land_plan_create")
+    best = None
+    for rep in range(3):
+        torch.cuda.synchronize()
+        barrier()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        with torch.cuda.stream(s_out):
+            e0.record()
+            for i in range(args.iters):
+                lib.b2e_land_plan_launch(plan, i + 1, C.c_void_p(s_out.cuda_stream))
+            e1.record()
+        torch.cuda.synchronize()
+        t = torch.tensor([e0.elapsed_time(e1) * 1e-3], dtype=torch.float64, device=dev)
+        if world > 1:
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        best = float(t.item()) if best is None else min(best, float(t.item()))
+    ok = int(seq_np[0]) == args.iters and bool((arr[rank * nb:(rank + 1) * nb] == src.cpu().numpy()).all())
+    if rank == 0:
+        per = nb * args.iters / best / 1e9
+        print(f"world={world} landing kernel                     : {best / args.iters * 1e6:7.1f} us per {nb / 1e6:.2f} MB, "
+              f"{per:5.1f} GB/s per rank, {per * world:6.1f} GB/s aggregate, data+seq {'ok' if ok else 'WRONG'}", flush=True)
+    lib.b2e_land_plan_destroy(plan)
     lib.b2e_host_unregister(arr.ctypes.data)
     lib.b2e_host_unregister(seq_np.ctypes.data)
     if world > 1:

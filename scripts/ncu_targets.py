@@ -65,7 +65,7 @@ if which in ("all", "humanoid"):
         hm.step((torch.rand((8192, 17), device=dev) * 0.8 - 0.4).float())
     torch.cuda.synchronize()
 if which in ("humanoid", "humanoid_warp", "humanoid_thread"):
-    impl = {"humanoid": "default", "humanoid_warp": "warp", "humanoid_thread": "thread"}[which]
+    impl = "thread" if which == "humanoid_thread" else "warp"
     hn = int(os.environ.get("B2E_NCU_N", "8192"))
     h = gymnasium_b200.make_vec("Humanoid-v5", num_envs=hn, copy=False, impl=impl)
     h.reset(seed=0)

@@ -286,30 +286,6 @@ def test_humanoid_info_masks_follow_syncvectorenv(output):
         np.testing.assert_array_equal(info["_final_obs"], te | tr)
 
 
-def test_lunarlander_grouping_is_scheduling_only():
-    """Envs are regrouped into warps by their contact / joint-limit state; that must never change results, and `order` must
-    be a permutation of the env indices."""
-    n, T = 3000, 260
-    envs = []
-    for grouping, lanes in ((4, 0), (0, 0), (1, 0), (32, 0), (0, 8)):
-        e = make("LunarLander-v3", n)
-        e._cfg.grouping, e._cfg.lanes_per_warp = grouping, lanes
-        e.reset(seed=17)
-        envs.append(e)
-    rs = np.random.default_rng(6)
-    for t in range(T):
-        a = rs.integers(0, 4, n)
-        outs = [e.step(a) for e in envs]
-        for o in outs[1:]:
-            for k in range(4):
-                np.testing.assert_array_equal(outs[0][k], o[k], err_msg=f"output {k} differs at step {t}")
-    slots = 32 * ((n + 31) // 32 + (n + 3) // 4)  # dense warps + sparse warps of 4 lanes (lander_group_slots)
-    order = envs[0]._s["order"].cpu().numpy()[:slots]
-    assert sorted(order[order >= 0].tolist()) == list(range(n))  # every env owns exactly one thread slot
-    work = envs[0]._s["work"].cpu().numpy()
-    assert work.min() >= 0 and work.max() <= 63 and len(np.unique(work)) > 3
-
-
 # ---------------------------------------------------------------------------------------------------------------------
 # Hopper-v5 (SURVEY 8f rank 4: the Humanoid solver generalised to another MuJoCo robot); checker = oracle/hopper.c
 @pytest.mark.parametrize("robot", ["Hopper-v5", "Walker2d-v5"])

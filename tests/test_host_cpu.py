@@ -37,9 +37,10 @@ def test_struct_layouts_match_header():
     assert C.sizeof(_lib.Batch) == 48
     assert C.sizeof(_lib.CartPoleCfg) == 24
     assert C.sizeof(_lib.FrozenLakeCfg) == 8 + 16 + 72
-    assert C.sizeof(_lib.LunarLanderCfg) == 40 and C.sizeof(_lib.LunarLanderState) == 104
+    assert C.sizeof(_lib.LunarLanderCfg) == 32 and C.sizeof(_lib.LunarLanderState) == 88
     assert _lib.load().b2e_lunarlander_state_words() == 12 * 16
-    assert C.sizeof(_lib.HumanoidCfg) == 88 and C.sizeof(_lib.HumanoidState) == 72
+    assert C.sizeof(_lib.HumanoidCfg) == 80 and C.sizeof(_lib.HumanoidState) == 72
+    assert C.sizeof(_lib.MjPlanarCfg) == 88 and C.sizeof(_lib.PipeSlot) == 88
 
 
 def test_argument_errors_do_not_need_a_gpu():
